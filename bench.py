@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
         --master-port 29500 bench.py --gpus 8 --steps 10 --warmup 3
     python bench.py --impl reference ...      # the reference's CPU arithmetic on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's results as DIR/*.npy
 
 Workload (default ``c4shard``): BASELINE configs[3] -- 10M chunks x 12 vecs x 1024-d fp32, row-sharded
 over 8 GPUs -- run as its per-GPU shard: every rank holds 1.25M chunks (15.36M vectors, 61.4 GB) and
@@ -53,10 +54,17 @@ WORKLOADS = {
 }
 
 
+def positive_int(text: str) -> int:
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {v}")
+    return v
+
+
 def parse_args() -> argparse.Namespace:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=positive_int, default=10, help="timed steps")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="c4shard", choices=sorted(WORKLOADS))
@@ -81,7 +89,29 @@ def parse_args() -> argparse.Namespace:
                     help="after the timed loop: the same step launched after 250 ms of idle, six times (is the scan slower inside a "
                          "loop of steps than timed alone?)")
     ap.add_argument("--filtered", action="store_true", help="also time metadata-filtered searches (both reference branches)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 or "
+                         "float64, at most 64 MB in all) so that two builds can be compared on identical seeded inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the GPU path; the reference arm times a host-side sample of the workload")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict[str, np.ndarray]) -> None:
+    """``out_dir/<name>.npy`` per array: float16/float32 as float32, everything else (float64, integer ids and
+    counts, exact below 2**53) as float64."""
+    conv = {name: a.astype(np.float32 if a.dtype in (np.float16, np.float32) else np.float64) for name, a in arrays.items()}
+    total = sum(a.nbytes for a in conv.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_MAX_BYTES}-byte limit")
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in conv.items():
+        np.save(d / f"{name}.npy", a)
 
 
 def resolve(args: argparse.Namespace) -> dict:
@@ -157,10 +187,10 @@ class ClockSampler:
 
 
 # ---- CPU arm: the reference's arithmetic (oracle port) on the host cores ----------------------------
-def cpu_reference_rate(w: dict, sample_chunks: int, reps: int, seed: int = 0) -> dict:
+def cpu_reference_rate(w: dict, sample_chunks: int, reps: int, seed: int = 0, warmup: int = 0) -> dict:
     """Time ``oracle.vector_search.blas_batch_topk`` (sgemm on all host cores -> cosine scaling ->
-    top-num_hits / group max / top-k) on a bounded sample of the workload and extrapolate linearly
-    in the number of vectors."""
+    top-num_hits / group max / top-k) on a bounded sample of the workload, ``reps`` timed runs after
+    ``warmup`` untimed ones, and extrapolate linearly in the number of vectors."""
     from oracle.vector_search import blas_batch_topk  # the ONLY product-side use of the oracle: the CPU baseline
     from synth import make_corpus, make_queries
 
@@ -179,6 +209,8 @@ def cpu_reference_rate(w: dict, sample_chunks: int, reps: int, seed: int = 0) ->
         # threads actually used: the BLAS pool after the limit (never more than the cores this process may run on)
         threads = min(want, max([i.get("num_threads", 1) for i in threadpool_info()] + [1])) if threadpool_info else want
         blas_batch_topk(E[: 1024 * w["vecs"]], w["vecs"], Q[:8], min(w["k"], 64), num_hits=w["num_hits"])  # warm BLAS
+        for _ in range(warmup):
+            blas_batch_topk(E, w["vecs"], Q, w["k"], num_hits=w["num_hits"])
         for _ in range(reps):
             t0 = time.perf_counter()
             blas_batch_topk(E, w["vecs"], Q, w["k"], num_hits=w["num_hits"])
@@ -195,13 +227,11 @@ def run_reference(args: argparse.Namespace, w: dict) -> None:
         return
     sample = args.cpu_sample_chunks or max(2048, min(w["chunks"], 16_384))
     t0 = time.perf_counter()
-    steps = max(1, args.steps)
-    r = cpu_reference_rate(w, sample, reps=max(1, args.warmup) + steps)
-    # reps include the warm-up iterations; the median is the per-step figure.
+    r = cpu_reference_rate(w, sample, reps=args.steps, warmup=args.warmup)   # the median of the timed steps is the per-step figure
     value = r["qps_over_10M"]
     line = {
         "impl": "reference", "metric": "queries/sec multi-vector MaxSim over 10M chunks", "value": value,
-        "unit": "queries/s (10M-chunk equivalent)", "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup,
+        "unit": "queries/s (10M-chunk equivalent)", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
         "ms_per_step": r["t_sample_s"] * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
         "dtype": "f32", "data": "synthetic",
         "config": {"workload": w["desc"], "batch": w["batch"], "k": w["k"], "num_hits": w["num_hits"],
@@ -278,10 +308,13 @@ def run_rerank(args: argparse.Namespace, w: dict) -> None:
         types = [np.r_[np.zeros(12, np.int32), np.ones(L - 12, np.int32)] for L in lens[:n]]
         torch.set_num_threads(len(os.sched_getaffinity(0)))
         orr.hf_logits(model, ids[:4], types[:4])     # first call pays thread-pool / allocator start-up
-        t0 = time.perf_counter(); orr.hf_logits(model, ids, types); dt = time.perf_counter() - t0
+        t0 = time.perf_counter()
+        for _ in range(args.steps):
+            orr.hf_logits(model, ids, types)
+        dt = (time.perf_counter() - t0) / args.steps
         v = n / dt
         print(json.dumps({"impl": "reference", "metric": "cross-encoder pairs/sec", "value": v, "unit": "pairs/s", "n_gpus": args.gpus,
-                          "steps": 1, "warmup": 0, "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "strong",
+                          "steps": args.steps, "warmup": 0, "ms_per_step": dt * 1e3, "higher_is_better": True, "scaling": "strong",
                           "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": {"workload": w["desc"]},
                           "cpu_baseline": {"value": v, "unit": "pairs/s", "cores": torch.get_num_threads(), "kind": "port",
                                            "sample": f"{n} pairs, transformers BertForSequenceClassification fp32"},
@@ -301,22 +334,25 @@ def run_rerank(args: argparse.Namespace, w: dict) -> None:
     if world > 1:
         dist.barrier()
     t0 = time.perf_counter()
-    _, scores = eng.score_tokens(ids, types)                  # host ids in -> host scores out
-    order = np.argsort(-scores.reshape(len(mine), n_c), axis=1, kind="stable")   # rerank_chunks' reorder
+    for _ in range(args.steps):
+        logits, scores = eng.score_tokens(ids, types)              # host ids in -> host scores out
+        order = np.argsort(-scores.reshape(len(mine), n_c), axis=1, kind="stable")   # rerank_chunks' reorder
     torch.cuda.synchronize()
-    dt = torch.tensor([time.perf_counter() - t0], dtype=torch.float64, device="cuda")
+    dt = torch.tensor([(time.perf_counter() - t0) / args.steps], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(dt, op=dist.ReduceOp.MAX)
+    if args.dump_outputs and rank == 0:   # this rank's queries (all of them on one GPU)
+        dump_outputs(args.dump_outputs, {"logits": logits, "scores": scores, "order": order})
     if rank == 0:
         total = n_q * n_c
         v = total / float(dt.item())
         tok = int(lens.sum())
-        line = {"metric": "cross-encoder pairs/sec", "value": v, "unit": "pairs/s", "n_gpus": world, "steps": 1, "warmup": 1,
+        line = {"metric": "cross-encoder pairs/sec", "value": v, "unit": "pairs/s", "n_gpus": world, "steps": args.steps, "warmup": 1,
                 "ms_per_step": float(dt.item()) * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
                 "dtype": "f16", "data": "synthetic (seeded weights, random token pairs, mean 200 tokens)",
                 "config": {"workload": w["desc"], "pairs": total, "tokens": tok, "parallelism": f"dp{world} over queries"},
                 "e2e": {"value": v, "unit": "pairs/s", "h2d_bytes_per_step": int(tok * 12 // world), "d2h_bytes_per_step": int(total * 8 // world)},
-                "gpu_launches": int(87 * np.ceil(tok / world / eng.max_tokens_per_call)), "reordered": int(order.shape[0])}
+                "gpu_launches": int(87 * np.ceil(tok / world / eng.max_tokens_per_call)) * args.steps, "reordered": int(order.shape[0])}
         # Tensor-pipe roofline of the whole forward (it is one fused sequence of GEMM-shaped kernels):
         # per layer 2*T*(4H^2 + 2HF) for the linears + 4*sum(L^2)*H for QK^T and PV (SURVEY 8d).
         Hh, Ff, Ly = 384, 1536, 12
@@ -487,6 +523,9 @@ def run_pool(args: argparse.Namespace, w: dict) -> None:
     ev1.record(); torch.cuda.synchronize()
     windows = [(w0, time.perf_counter())]
     ms = ev0.elapsed_time(ev1) / args.steps
+    if args.dump_outputs:   # a seeded sample of the pooled rows: all of them (S x 1024) would exceed the dump limit
+        pick = np.sort(np.random.default_rng(0).choice(S, size=min(S, 8192), replace=False))
+        dump_outputs(args.dump_outputs, {"pooled": outd[torch.from_numpy(pick).to(dev)].cpu().numpy(), "pooled_rows": pick})
     pooled_rows = int((re_ - rb).sum())
     alg_bytes = pooled_rows * d * 4 + S * d * 2 + S * 8
     t0 = time.perf_counter()
@@ -637,6 +676,9 @@ def main() -> None:  # noqa: PLR0915
     ev1.record()
     barrier()
     windows.append((w0, time.perf_counter()))
+    if args.dump_outputs and rank == 0:   # the merged result of the last timed step: every rank holds the same one
+        sim, chunk, count, status = (t.cpu().numpy() for t in out)
+        dump_outputs(args.dump_outputs, {"sim": sim, "chunk": chunk, "count": count, "status": status})
     ms_total = ev0.elapsed_time(ev1)
     t = torch.tensor([ms_total], dtype=torch.float64, device=device)
     if world > 1:
