@@ -57,7 +57,7 @@ def build(force: bool = False, verbose: bool = False) -> Path:
             if not force and not is_stale():
                 return LIB_PATH
             tmp = LIB_PATH.with_suffix(f".so.tmp{os.getpid()}")
-            extra = os.environ.get("RL_NVCC_EXTRA", "").split()   # A/B builds on the GPU box (e.g. -DRL_EPI_SIGN=0)
+            extra = os.environ.get("RL_NVCC_EXTRA", "").split()   # extra nvcc flags (e.g. -Xptxas=-warn-spills)
             cmd = [nvcc, *NVCC_FLAGS, *extra, "-o", str(tmp), *[str(s) for s in sources()]]
             if verbose:
                 cmd.insert(1, "-Xptxas=-v")

@@ -489,6 +489,3 @@ extern "C" int rl_maxsim_unfiltered_bound(const rl_scan_params* p, const void* w
   RL_CUDA_CHECK(cudaGetLastError());
   return RL_OK;
 }
-
-// (not declared in the public header: a build-time diagnostic used by tools/probe_attrs.py)
-extern "C" int rl_debug_scan_kernel_attrs(int which, int* out) { return rl::debug_scan_kernel_attrs(which, out); }

@@ -34,9 +34,6 @@ namespace {
 
 using namespace tc;
 
-#ifndef RL_EPI_SIGN
-#define RL_EPI_SIGN 1   // emit-mode epilogue: sign collector (FFMA + funnel shift) instead of FMUL + FSETP + SEL
-#endif
 constexpr int kTileM = 128;           // corpus rows per tile (UMMA M)
 constexpr int kSliceK = 64;           // fp16 elements per K slice = one 128-byte swizzle row
 constexpr int kMaxQ = 256;            // queries per pass (UMMA N <= 256)
@@ -50,6 +47,7 @@ constexpr int kMaxStages = 8;
 constexpr int kABytes = kTileM * 128;  // 16 KB per stage
 constexpr uint32_t kSmemBudget = 222 * 1024;
 constexpr int kPrefetchItems = 6;      // L2 prefetch distance in K-slice items (6 x 32 KB per SM)
+constexpr int kPrefetchPairs = kPrefetchItems / 2;   // the same distance for the fast fp32 loader, in pairs of items
 constexpr int kListCap = 1024;         // staged hit records (12 KB)
 constexpr int kFlushFirst = 192;       // first flush early: it feeds the histogram that tightens the thresholds
 constexpr int kFlushAt = 512;          // later flushes: once this many hits are waiting (or at the end)
@@ -61,15 +59,13 @@ struct TcArgs {
   const __half* qimg;     // [n_ks][nq][64] fp16, rows pre-swizzled
   const float* q_scale;   // [B] key = acc * q_scale[b] (+ bias)
   const float* row_stats; // [2] max norm, max |element|
-  int nq;                 // padded #queries of a FULL group (multiple of 16; kMaxQ when n_groups > 1)
-  int n_groups;           // query groups of kMaxQ walked per corpus tile (B <= n_groups * kMaxQ)
+  int nq;                 // padded #queries of a FULL group (multiple of 16; kMaxQ when par_groups > 1)
   int nq_last;            // padded #queries of the last group
   int par_groups;         // > 1: group-parallel -- CTA c serves query group c % par_groups of the tiles of lane c / par_groups
   int n_ks;               // K slices
   int stages;
   int tmem_cols;          // allocated TMEM columns (power of two >= 2 * buf_cols)
   int buf_cols;           // columns per accumulator buffer (nq rounded up to 32)
-  int pf_pairs;           // fast fp32 loader: L2 prefetch distance in pairs of K-slice items (0: no prefetch)
   int tma_rows;           // fp16 storage: 1 = corpus tiles come through the tensor map (no loader warps)
 };
 
@@ -108,14 +104,11 @@ struct SmemLayout {
 };
 
 __host__ __device__ inline uint32_t stage_bytes(int nq) { return kABytes + (uint32_t)nq * 128u; }
-// One query group (B <= 256): thresholds, scales, histogram origin / bin width, the staged histogram and the
-// per-query counters all live in shared memory.  Several groups per tile (B > 256, configs[2]): only
-// thresholds, scales and counters (the histogram is updated with global atomics at hit time, its origin
-// and bin width are read from global memory there) -- that keeps four pipeline stages.
-__host__ __device__ inline uint32_t tail_bytes(int n_groups) {
-  const uint32_t qt = (uint32_t)n_groups * kMaxQ;
-  const uint32_t per_q = n_groups > 1 ? 4u * 4u : 6u * 4u + (uint32_t)kHistBins * 2u;
-  return (2 * kMaxStages + 4) * 8 + 16 + qt * per_q + 16 + kListCap * 12;
+// Per query of the CTA's group: threshold, scale, histogram origin / bin width, the staged histogram and the
+// counters, all in shared memory.
+__host__ __device__ inline uint32_t tail_bytes() {
+  const uint32_t per_q = 6u * 4u + (uint32_t)kHistBins * 2u;
+  return (2 * kMaxStages + 4) * 8 + 16 + kMaxQ * per_q + 16 + kListCap * 12;
 }
 
 // PAIR: two CTAs of a cluster (an SM pair) issue one cta_group::2 MMA (M = 256: 128 rows per CTA) and
@@ -125,17 +118,15 @@ __host__ __device__ inline uint32_t tail_bytes(int n_groups) {
 template <int METRIC, bool PAIR, bool EF16>
 __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUtensorMap tmE, const TcArgs t) {
   extern __shared__ unsigned char smem_dyn[];
-  // Group-parallel mode (B > 256, the default): the CTAs of a "lane" -- par_groups consecutive CTAs -- walk the
-  // SAME corpus tiles at the same time, one 256-query group each.  The first of them pulls a tile in from
-  // HBM, the others find it in L2 microseconds later, so HBM sees the corpus once; every CTA keeps the
-  // single-group shared-memory state.  (Walking the groups one after the other inside a CTA -- n_groups > 1 --
-  // puts a 512 KB x 148 = 76 MB reuse distance between the passes over a tile: the re-reads then miss L2.)
+  // Group-parallel mode (B > 256): the CTAs of a "lane" -- par_groups consecutive CTAs -- walk the SAME corpus
+  // tiles at the same time, one 256-query group each.  The first of them pulls a tile in from HBM, the others
+  // find it in L2 microseconds later, so HBM sees the corpus once.
   const int P = t.par_groups > 1 ? t.par_groups : 1;
   const int pg = P > 1 ? (int)((PAIR ? blockIdx.x >> 1 : blockIdx.x) % (unsigned)P) : 0;
   ScanArgs a = t.a;
   const float* q_scale_g = t.q_scale;
   const __half* qimg_g = t.qimg;
-  int nqF = t.nq, nqL = t.nq_last;       // padded width of a full group / of the last group this CTA serves
+  int nq = t.nq;                         // padded width of the group this CTA serves
   if (P > 1) {
     const int q0p = pg * kMaxQ;
     a.B = min(kMaxQ, t.a.B - q0p);
@@ -146,7 +137,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     a.ghist += (size_t)q0p * kHistBins;
     q_scale_g += q0p;
     qimg_g += (size_t)pg * t.n_ks * kMaxQ * kSliceK;
-    nqF = nqL = (pg == P - 1) ? t.nq_last : t.nq;
+    nq = (pg == P - 1) ? t.nq_last : t.nq;
   }
   // 1024-byte alignment for the 128B-swizzled tiles.
   // (pointer arithmetic on the __shared__ array keeps the address space known: LDS/STS, not generic LD/ST)
@@ -159,22 +150,18 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
   s.tmem_full = s.empty + kMaxStages;
   s.tmem_empty = s.tmem_full + 2;
   s.tmem_ptr = reinterpret_cast<uint32_t*>(s.tmem_empty + 2);
-  const int G = t.n_groups;
-  const bool multi = G > 1;
-  const int QT = G * kMaxQ;            // query slots of this launch
+  // Per-query arrays.  Their pitch goes through an opaque move: with compile-time offsets ptxas keeps one pointer
+  // per array live across every warp role, and the dot / l2 instantiations spill at the 128-register cap.
+  int qp = kMaxQ;
+  asm volatile("" : "+r"(qp));
   s.thr = reinterpret_cast<float*>(s.tmem_ptr + 4);
-  s.cs = s.thr + QT;
-  if (!multi) {
-    s.thr0 = s.cs + QT;
-    s.inv_w = s.thr0 + QT;
-    s.hist = reinterpret_cast<uint32_t*>(s.inv_w + QT);
-    s.cnt = reinterpret_cast<int*>(s.hist + QT * kHistBins / 2);
-  } else {
-    s.thr0 = nullptr; s.inv_w = nullptr; s.hist = nullptr;
-    s.cnt = reinterpret_cast<int*>(s.cs + QT);
-  }
-  s.basev = s.cnt + QT;
-  s.list_n = s.basev + QT;
+  s.cs = s.thr + qp;
+  s.thr0 = s.cs + qp;
+  s.inv_w = s.thr0 + qp;
+  s.hist = reinterpret_cast<uint32_t*>(s.inv_w + qp);
+  s.cnt = reinterpret_cast<int*>(s.hist + qp * kHistBins / 2);
+  s.basev = s.cnt + qp;
+  s.list_n = s.basev + qp;
   s.list = reinterpret_cast<uint32_t*>(s.list_n + 4);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -189,10 +176,6 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     const int64_t unit = first + tile * stride;
     return PAIR ? 2 * unit + rank : unit;
   };
-  // B > 256: every corpus tile is walked once per query group, back to back (group-minor order), so the
-  // re-reads of the tile hit L2 and HBM sees the corpus once.  "Virtual tile" v = tile * n_groups + group.
-  const int G0 = t.n_groups;
-  const int64_t v_tiles = my_tiles * G0;
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < t.stages; ++i) {
@@ -207,17 +190,14 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     }
     fence_barrier_init();
   }
-  for (int i = threadIdx.x; i < QT; i += blockDim.x) {
+  for (int i = threadIdx.x; i < kMaxQ; i += blockDim.x) {
     s.thr[i] = (i < a.B && !a.dump_mode) ? a.thr[i] : __int_as_float(0x7f800000);  // +inf: never emit
     s.cs[i] = (i < a.B) ? q_scale_g[i] : 0.f;
     s.cnt[i] = 0;
-    if (!multi) {
-      s.thr0[i] = s.thr[i];
-      s.inv_w[i] = (i < a.B && !a.dump_mode) ? a.hist_inv_w[i] : 0.f;
-    }
+    s.thr0[i] = s.thr[i];
+    s.inv_w[i] = (i < a.B && !a.dump_mode) ? a.hist_inv_w[i] : 0.f;
   }
-  if (!multi)
-    for (int i = threadIdx.x; i < kMaxQ * kHistBins / 2; i += blockDim.x) s.hist[i] = 0u;
+  for (int i = threadIdx.x; i < kMaxQ * kHistBins / 2; i += blockDim.x) s.hist[i] = 0u;
   if (threadIdx.x == 0) { s.list_n[0] = 0; s.list_n[1] = 0; }
   if (warp == kMmaWarp) {
     if (PAIR) tmem_alloc_2cta(s.tmem_ptr, (uint32_t)t.tmem_cols);
@@ -235,7 +215,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
                                      t.row_stats[3] == 0.f));   // (the host only allows fp16 storage when this holds)
 
   // fp32 loader fast path (uniform): whole K slices in pairs, one query group per CTA, no per-row scale in the loader
-  const bool fast_f32 = !EF16 && G0 == 1 && a.d % kSliceK == 0 && (t.n_ks & 1) == 0 && a.ld * 64 < (int64_t(1) << 32) &&
+  const bool fast_f32 = !EF16 && a.d % kSliceK == 0 && (t.n_ks & 1) == 0 && a.ld * 64 < (int64_t(1) << 32) &&
                         (METRIC != RL_METRIC_COSINE || cos_noscale);
   if (EF16 && t.tma_rows && warp >= kFirstLoaderWarp) {
     // fp16 storage through the tensor map: the producer thread issues one cp.async.bulk.tensor per K slice and the
@@ -249,16 +229,16 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     const __half* Eh = reinterpret_cast<const __half*>(a.E);
     // (fp16-stored rows are used as they are: no global power-of-two scale -- it only guards the fp32 -> fp16
     // conversion against overflow -- and the query scale is built without it, see query_image_kernel)
-    const int64_t total_items = v_tiles * t.n_ks;
+    const int64_t total_items = my_tiles * t.n_ks;
     const size_t pitch32_bytes = (size_t)a.ld * 32 * sizeof(__half);
     const size_t slice_bytes = kSliceK * sizeof(__half);
     uint4 ring[4][4];
     int64_t ld_tile = 0;
     int ld_ks = 0, ld_rows = 0;
     const unsigned char* ld_ptr = nullptr;
-    auto ld_set_tile = [&]() {   // ld_tile / pf_tile count virtual tiles
-      if (ld_tile < v_tiles && ord_of(ld_tile / G0) < a.n_mode_blocks) {
-        const int64_t blk = mode_block_index(a, ord_of(ld_tile / G0));
+    auto ld_set_tile = [&]() {
+      if (ld_tile < my_tiles && ord_of(ld_tile) < a.n_mode_blocks) {
+        const int64_t blk = mode_block_index(a, ord_of(ld_tile));
         const int64_t rem = a.n_rows - blk * kTileM;
         ld_rows = rem < kTileM ? (int)rem : kTileM;
         ld_ptr = reinterpret_cast<const unsigned char*>(Eh + (size_t)(blk * kTileM + r0) * a.ld + j * 8);
@@ -269,9 +249,9 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     int64_t pf_tile = 0;
     int pf_ks = 0, pf_rows = 0;
     const unsigned char* pf_ptr = nullptr;
-    auto pf_set_tile = [&]() {   // only the first group's pass over a tile comes from HBM
-      if (pg == 0 && pf_tile < v_tiles && pf_tile % G0 == 0 && ord_of(pf_tile / G0) < a.n_mode_blocks) {
-        const int64_t blk = mode_block_index(a, ord_of(pf_tile / G0));
+    auto pf_set_tile = [&]() {   // only the first group's CTA of a lane prefetches
+      if (pg == 0 && pf_tile < my_tiles && ord_of(pf_tile) < a.n_mode_blocks) {
+        const int64_t blk = mode_block_index(a, ord_of(pf_tile));
         const int64_t rem = a.n_rows - blk * kTileM;
         pf_rows = rem < kTileM ? (int)rem : kTileM;
         pf_ptr = reinterpret_cast<const unsigned char*>(Eh + (size_t)(blk * kTileM + (lt & 127)) * a.ld);
@@ -333,7 +313,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
       if (item + 3 < total_items) process(ring[3]);
     }
   } else if (warp >= kFirstLoaderWarp && fast_f32) {
-    // ===== corpus loaders, fp32 storage, FAST PATH (d % 128 == 0, one query group per CTA, no per-row scale) =====
+    // ===== corpus loaders, fp32 storage, FAST PATH (d % 128 == 0, no per-row scale) =====
     // Same data movement as the generic loader below -- HBM fp32 -> registers (two K-slice items = 64 KB per SM in
     // flight) -> cvt.rn.f16x2 -> 128B-swizzled smem tile, L2 prefetch kPrefetchItems ahead -- with the bookkeeping
     // cut down.  ncu's source view of the generic loop showed ~155 SASS instructions per item and warp (three
@@ -373,7 +353,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     Cursor pf{0, 0u, 0, nullptr};
     auto pf_set_tile = [&]() {
       pf.rows = 0;
-      if (pg == 0 && t.pf_pairs > 0 && pf.tile < my_tiles) {
+      if (pg == 0 && pf.tile < my_tiles) {
         const int64_t ord = ord_of(pf.tile);
         if (ord < a.n_mode_blocks) {
           const int64_t blk = mode_block_index(a, ord);
@@ -428,7 +408,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
 
     ld_set_tile();
     pf_set_tile();
-    for (int i = 0; i < t.pf_pairs + 1; ++i) pf_pair();   // the load cursor starts one pair ahead of the stores
+    for (int i = 0; i < kPrefetchPairs + 1; ++i) pf_pair();   // the load cursor starts one pair ahead of the stores
     issue(ringA, ld.rows, ld.ptr);
     issue(ringB, ld.rows, ld.ptr + 256);
     for (int64_t item = 0; item < total_items; item += 2) {
@@ -453,7 +433,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     // Rows are converted without a multiply when no scaling is needed (normalised corpora: the
     // cosine 1/|e| then moves to the epilogue, which has slack; dot/l2: the global scale is 1).
     const bool noscale = (METRIC == RL_METRIC_COSINE) ? cos_noscale : (gscale == 1.f);
-    const int64_t total_items = v_tiles * t.n_ks;
+    const int64_t total_items = my_tiles * t.n_ks;
     float4 ring[2][8];
     float rs[8];
 
@@ -464,9 +444,9 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     int64_t ld_tile = 0;
     int ld_ks = 0, ld_rows = 0;
     const unsigned char* ld_ptr = nullptr;                 // row r0 of the tile, column c4*4 + ld_ks*64
-    auto ld_set_tile = [&]() {   // ld_tile / pf_tile / st_tile count virtual tiles
-      if (ld_tile < v_tiles && ord_of(ld_tile / G0) < a.n_mode_blocks) {
-        const int64_t blk = mode_block_index(a, ord_of(ld_tile / G0));
+    auto ld_set_tile = [&]() {
+      if (ld_tile < my_tiles && ord_of(ld_tile) < a.n_mode_blocks) {
+        const int64_t blk = mode_block_index(a, ord_of(ld_tile));
         const int64_t rem = a.n_rows - blk * kTileM;
         ld_rows = rem < kTileM ? (int)rem : kTileM;
         ld_ptr = reinterpret_cast<const unsigned char*>(a.E + (size_t)(blk * kTileM + r0) * a.ld + c4 * 4);
@@ -478,9 +458,9 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     int64_t pf_tile = 0;
     int pf_ks = 0, pf_rows = 0;
     const unsigned char* pf_ptr = nullptr;
-    auto pf_set_tile = [&]() {   // only the first group's pass over a tile comes from HBM
-      if (pg == 0 && pf_tile < v_tiles && pf_tile % G0 == 0 && ord_of(pf_tile / G0) < a.n_mode_blocks) {
-        const int64_t blk = mode_block_index(a, ord_of(pf_tile / G0));
+    auto pf_set_tile = [&]() {   // only the first group's CTA of a lane prefetches
+      if (pg == 0 && pf_tile < my_tiles && ord_of(pf_tile) < a.n_mode_blocks) {
+        const int64_t blk = mode_block_index(a, ord_of(pf_tile));
         const int64_t rem = a.n_rows - blk * kTileM;
         pf_rows = rem < kTileM ? (int)rem : kTileM;
         pf_ptr = reinterpret_cast<const unsigned char*>(a.E + (size_t)(blk * kTileM + (lt >> 1)) * a.ld + (lt & 1) * 32);
@@ -532,8 +512,8 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     auto fetch_scales = [&](int64_t tile) {
 #pragma unroll
       for (int i = 0; i < 8; ++i) rs[i] = (METRIC == RL_METRIC_COSINE) ? 0.f : gscale;
-      if (METRIC == RL_METRIC_COSINE && !noscale && tile < v_tiles && ord_of(tile / G0) < a.n_mode_blocks) {
-        const int64_t blk = mode_block_index(a, ord_of(tile / G0));
+      if (METRIC == RL_METRIC_COSINE && !noscale && tile < my_tiles && ord_of(tile) < a.n_mode_blocks) {
+        const int64_t blk = mode_block_index(a, ord_of(tile));
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
           const int64_t row = blk * kTileM + r0 + 16 * i;
@@ -592,40 +572,36 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
   } else if (warp == kQWarp) {
     // ===== query producer: bulk-copy the pre-swizzled fp16 K slice of all queries (UMMA B operand) =====
     if (lane == 0) {
-      // Group g's image starts g * (n_ks * kMaxQ * kSliceK) halves into qimg; inside a group the K slices of
-      // its nq_g queries follow each other (nq_g * 128 bytes each).
-      const size_t group_bytes = (size_t)t.n_ks * kMaxQ * kSliceK * sizeof(__half);
-      const int64_t total_items = v_tiles * t.n_ks;
-      int ks = 0, stage = 0, g = 0;
+      // The K slices of the group's nq queries follow each other in its image (nq * 128 bytes each).
+      const uint32_t slice_bytes_q = (uint32_t)nq * 128u;
+      const uint32_t qbytes = PAIR ? slice_bytes_q / 2 : slice_bytes_q;   // PAIR: this CTA's half of them
+      const unsigned char* qsrc = reinterpret_cast<const unsigned char*>(qimg_g) + (PAIR ? (size_t)rank * qbytes : 0);
+      const int64_t total_items = my_tiles * t.n_ks;
+      int ks = 0, stage = 0;
       uint32_t phase = 0;
       // fp16 storage, tensor-map mode: this thread also brings the corpus tile -- row0 of the current tile (-1: this
       // CTA has no block for the tile, nothing is loaded and the epilogue ignores the accumulator) and of the
       // next one, whose slices are prefetched into L2 one tile (n_ks slices = 256 KB per SM at d = 1024) ahead.
       const bool tma_rows = EF16 && t.tma_rows;
-      int64_t vt = 0;
+      int64_t tile = 0;
       int row0 = -1, row0_next = -1;
       auto tile_row0 = [&](int64_t v) -> int {
-        if (v >= v_tiles) return -1;
-        const int64_t ord = ord_of(v / G0);
+        if (v >= my_tiles) return -1;
+        const int64_t ord = ord_of(v);
         return ord < a.n_mode_blocks ? (int)(mode_block_index(a, ord) * kTileM) : -1;
       };
       if (tma_rows) { row0 = tile_row0(0); row0_next = tile_row0(1); }
       for (int64_t item = 0; item < total_items; ++item) {
-        const uint32_t slice_bytes_q = (uint32_t)(g == G0 - 1 ? nqL : nqF) * 128u;   // one K slice of the group's queries
-        const uint32_t qbytes = PAIR ? slice_bytes_q / 2 : slice_bytes_q;                    // PAIR: this CTA's half of them
-        const unsigned char* qsrc = reinterpret_cast<const unsigned char*>(qimg_g) + (size_t)g * group_bytes +
-                                    (PAIR ? (size_t)rank * qbytes : 0);
         mbar_wait(&s.empty[stage], phase ^ 1u);
         const bool load_a = tma_rows && row0 >= 0;
         mbar_arrive_expect_tx(&s.full[stage], qbytes + (load_a ? (uint32_t)kABytes : 0u));
         if (load_a) tma_load_tile(s.stage_base + (size_t)stage * sbytes, &tmE, ks * kSliceK, row0, &s.full[stage]);
         bulk_g2s(s.stage_base + (size_t)stage * sbytes + kABytes, qsrc + (size_t)ks * slice_bytes_q, qbytes,
                  &s.full[stage]);
-        if (tma_rows && row0_next >= 0 && pg == 0 && g == 0) tma_prefetch_tile(&tmE, ks * kSliceK, row0_next);
+        if (tma_rows && row0_next >= 0 && pg == 0) tma_prefetch_tile(&tmE, ks * kSliceK, row0_next);
         if (++ks == t.n_ks) {
           ks = 0;
-          if (++g == G0) g = 0;
-          if (tma_rows) { ++vt; row0 = row0_next; row0_next = tile_row0(vt + 1); }
+          if (tma_rows) { ++tile; row0 = row0_next; row0_next = tile_row0(tile + 1); }
         }
         if (++stage == t.stages) { stage = 0; phase ^= 1u; }
       }
@@ -638,7 +614,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
       if (lane == 0) {
         int stage = 0;
         uint32_t phase = 0;
-        const int64_t total_items = v_tiles * t.n_ks;
+        const int64_t total_items = my_tiles * t.n_ks;
         for (int64_t item = 0; item < total_items; ++item) {
           mbar_wait(&s.full[stage], phase);
           fence_proxy_async();
@@ -647,13 +623,10 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
         }
       }
     } else if (lane == 0) {
-      const uint32_t idesc_full = make_idesc_f16(PAIR ? 2 * kTileM : kTileM, nqF);
-      const uint32_t idesc_last = make_idesc_f16(PAIR ? 2 * kTileM : kTileM, nqL);
-      int stage = 0, g = 0;
+      const uint32_t idesc = make_idesc_f16(PAIR ? 2 * kTileM : kTileM, nq);
+      int stage = 0;
       uint32_t phase = 0;
-      for (int64_t tile = 0; tile < v_tiles; ++tile) {   // virtual tiles: (corpus tile, query group)
-        const uint32_t idesc = g == G0 - 1 ? idesc_last : idesc_full;
-        if (++g == G0) g = 0;
+      for (int64_t tile = 0; tile < my_tiles; ++tile) {
         const int buf = (int)(tile & 1);
         if (PAIR) mbar_wait_cluster(&s.tmem_empty[buf], (uint32_t)(((tile >> 1) & 1) ^ 1));
         else mbar_wait(&s.tmem_empty[buf], (uint32_t)(((tile >> 1) & 1) ^ 1));
@@ -687,12 +660,8 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
     // ===== epilogue warps 0..3: TMEM -> registers -> key -> dump / threshold + emit =====
     const int q = warp;  // TMEM lane quarter
     bool flushed_once = false;
-    int g = 0;           // query group of the current virtual tile
-    for (int64_t vt = 0; vt < v_tiles; ++vt) {
-      const int64_t tile = multi ? vt / G0 : vt;   // corpus tile
-      const int q0 = g * kMaxQ;                    // first query slot of this group
-      const int nq_g = g == G0 - 1 ? nqL : nqF;
-      const int buf = (int)(vt & 1);
+    for (int64_t tile = 0; tile < my_tiles; ++tile) {
+      const int buf = (int)(tile & 1);
       const int64_t ord = ord_of(tile);
       const bool has_block = ord < a.n_mode_blocks;
       const int64_t blk = has_block ? mode_block_index(a, ord) : 0;
@@ -708,7 +677,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
       }
       const float bias = (METRIC == RL_METRIC_L2 && valid) ? -a.sq_norm[row] : 0.f;
       const float lane_scale = (METRIC == RL_METRIC_COSINE && cos_noscale && valid) ? __ldg(a.inv_norm + row) : 1.f;
-      mbar_wait(&s.tmem_full[buf], (uint32_t)((vt >> 1) & 1));
+      mbar_wait(&s.tmem_full[buf], (uint32_t)((tile >> 1) & 1));
       tc_fence_after();
       const uint32_t taddr0 = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(buf * t.buf_cols);
       // Two register buffers: the TMEM load of chunk c+1 is in flight while chunk c is processed.
@@ -716,7 +685,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
         if (a.dump_mode) {
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
-            const int col = q0 + c0 + j;
+            const int col = c0 + j;
             if (col < a.B) {
               float key = __uint_as_float(v[j]);
               if (METRIC != RL_METRIC_COSINE) key = fmaf(key, s.cs[col], bias);
@@ -727,56 +696,40 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
         } else {
           // Two instructions per accumulator: the sign of  acc * scale - thr  (one FFMA; dot / l2: FFMA + FADD) is
           // shifted into a bit collector with one funnel shift -- element j ends up at bit 31 - j, set when the
-          // key is BELOW its threshold.  (Was FMUL + FSETP + SEL + an occasional IADD3: 3.5 per accumulator, a
-          // quarter of the SM's issued instructions.)  For cosine the FFMA rounds once, so a key whose rounded
-          // product equals thr while the exact product lies below it no longer counts as a hit; thr sits 2 eps
-          // (~1e-3) under anything the selection needs, a rounding step is 6e-8.
-#if RL_EPI_SIGN
+          // key is BELOW its threshold (FMUL + FSETP + SEL took 3.5 per accumulator, DESIGN.md 3.1).  For cosine
+          // the FFMA rounds once, so a key whose rounded product equals thr while the exact product lies below it
+          // does not count as a hit; thr sits 2 eps (~1e-3) under anything the selection needs, a rounding step is 6e-8.
           uint32_t below = 0;
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             const float acc = __uint_as_float(v[j]);
             float tkey;
-            if (METRIC != RL_METRIC_COSINE) tkey = fmaf(acc, s.cs[q0 + c0 + j], bias) - s.thr[q0 + c0 + j];
-            else tkey = fmaf(acc, lane_scale, -s.thr[q0 + c0 + j]);
+            if (METRIC != RL_METRIC_COSINE) tkey = fmaf(acc, s.cs[c0 + j], bias) - s.thr[c0 + j];
+            else tkey = fmaf(acc, lane_scale, -s.thr[c0 + j]);
             below = __funnelshift_l(__float_as_uint(tkey), below, 1);
           }
           uint32_t mask = __brev(~below);   // bit j set <=> key j at or above its threshold
-#else
-          uint32_t mask = 0;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            float key = __uint_as_float(v[j]);
-            if (METRIC != RL_METRIC_COSINE) key = fmaf(key, s.cs[q0 + c0 + j], bias);
-            else key *= lane_scale;
-            if (key >= s.thr[q0 + c0 + j]) mask |= 1u << j;
-          }
-#endif
           if (masked_alive) {   // (only with RL_FLAG_COUNT_UNFILTERED on a filtered scan)
             uint32_t extra = mask;
             while (extra != 0) {
               const int j = __ffs(extra) - 1;
               extra &= extra - 1;
-              atomicAdd(a.cnt_all + q0 + c0 + j, 1);
+              atomicAdd(a.cnt_all + c0 + j, 1);
             }
           }
           if (!valid) mask = 0;
           while (mask != 0) {  // rare: a few hits per tile; picks v[j] with a register select tree
             const int j = __ffs(mask) - 1;
             mask &= mask - 1;
-            const int col = q0 + c0 + j;
+            const int col = c0 + j;
             float key = __uint_as_float(select32(v, j));
             if (METRIC != RL_METRIC_COSINE) key = fmaf(key, s.cs[col], bias);
             else key *= lane_scale;
             // Stage the hit in shared memory (one returning atomic for the slot; the histogram update
             // does not wait); per-query ranks and global slots are handed out in bulk at the flush.
             const int pos = atomicAdd(&s.list_n[0], 1);
-            if (!multi) {
-              const int hb = col * kHistBins + hist_bin(key, s.thr0[col], s.inv_w[col]);
-              atomicAdd(&s.hist[hb >> 1], 1u << ((hb & 1) * 16));
-            } else {   // several groups per tile: the histogram lives in global memory only (fire-and-forget RED)
-              atomicAdd(a.ghist + (size_t)col * kHistBins + hist_bin(key, __ldg(a.thr + col), __ldg(a.hist_inv_w + col)), 1);
-            }
+            const int hb = col * kHistBins + hist_bin(key, s.thr0[col], s.inv_w[col]);
+            atomicAdd(&s.hist[hb >> 1], 1u << ((hb & 1) * 16));
             if (pos < kListCap) {
               s.list[pos * 3 + 0] = (uint32_t)col;
               s.list[pos * 3 + 1] = __float_as_uint(key);
@@ -790,20 +743,20 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
       uint32_t va[32], vb[32];
       tmem_ld32_async(taddr0, va);
       tmem_ld_wait(va);
-      for (int c0 = 0; c0 < nq_g; c0 += 64) {
-        const bool has_b = c0 + 32 < nq_g;
+      for (int c0 = 0; c0 < nq; c0 += 64) {
+        const bool has_b = c0 + 32 < nq;
         if (has_b) tmem_ld32_async(taddr0 + (uint32_t)(c0 + 32), vb);
         process_chunk(c0, va);
         if (has_b) {
           tmem_ld_wait(vb);
-          if (c0 + 64 < nq_g) tmem_ld32_async(taddr0 + (uint32_t)(c0 + 64), va);
+          if (c0 + 64 < nq) tmem_ld32_async(taddr0 + (uint32_t)(c0 + 64), va);
           process_chunk(c0 + 32, vb);
-          if (c0 + 64 < nq_g) tmem_ld_wait(va);
+          if (c0 + 64 < nq) tmem_ld_wait(va);
         }
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) {  // TMEM buffer is free for virtual tile + 2 (the leader CTA's barrier counts both epilogues)
+      if (lane == 0) {  // TMEM buffer is free for tile + 2 (the leader CTA's barrier counts both epilogues)
         if (PAIR && rank != 0) mbar_arrive_remote(mapa_u32(&s.tmem_empty[buf], 0));
         else mbar_arrive(&s.tmem_empty[buf]);
       }
@@ -815,7 +768,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
         epi_bar_sync();
         const int n_all = s.list_n[0];
         epi_bar_sync();
-        const bool last = vt + 1 == v_tiles;
+        const bool last = tile + 1 == my_tiles;
         const bool do_flush = n_all >= (flushed_once ? kFlushAt : kFlushFirst) || (last && n_all > 0);
         if (do_flush) {
           flushed_once = true;
@@ -825,21 +778,19 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
             s.list[e * 3 + 0] = (uint32_t)col | ((uint32_t)atomicAdd(&s.cnt[col], 1) << 16);
           }
           epi_bar_sync();
-          for (int col = et; col < QT; col += kNumEpiWarps * 32) {
+          for (int col = et; col < kMaxQ; col += kNumEpiWarps * 32) {
             const int c = s.cnt[col];
             if (c > 0) {
               s.basev[col] = atomicAdd(a.cand_cnt + col, c);
               s.cnt[col] = 0;
             }
           }
-          if (!multi) {
-            for (int w = et; w < kMaxQ * kHistBins / 2; w += kNumEpiWarps * 32) {
-              const uint32_t h = s.hist[w];
-              if (h != 0u) {
-                if (h & 0xFFFFu) atomicAdd(a.ghist + 2 * w, (int)(h & 0xFFFFu));
-                if (h >> 16) atomicAdd(a.ghist + 2 * w + 1, (int)(h >> 16));
-                s.hist[w] = 0u;
-              }
+          for (int w = et; w < kMaxQ * kHistBins / 2; w += kNumEpiWarps * 32) {
+            const uint32_t h = s.hist[w];
+            if (h != 0u) {
+              if (h & 0xFFFFu) atomicAdd(a.ghist + 2 * w, (int)(h & 0xFFFFu));
+              if (h >> 16) atomicAdd(a.ghist + 2 * w + 1, (int)(h >> 16));
+              s.hist[w] = 0u;
             }
           }
           epi_bar_sync();
@@ -856,423 +807,7 @@ __global__ void __maxnreg__(128) scan_tcgen05_kernel(const __grid_constant__ CUt
         if ((do_flush || periodic) && !last) {
           // Threshold refresh: the highest bin edge with >= sel_count candidates at or above it (all
           // CTAs' hits so far) bounds the sel_count-th best key from below; emit from 2 eps under it.
-          // (Several groups per tile: the group just processed is refreshed -- each group every 16 tiles.)
-          const int c_lo = multi ? q0 : 0, c_hi = multi ? min(a.B, q0 + kMaxQ) : a.B;
-          for (int col = c_lo + et; col < c_hi; col += kNumEpiWarps * 32) {
-            const int4* gh = reinterpret_cast<const int4*>(a.ghist + (size_t)col * kHistBins);
-            int cnts[kHistBins];
-#pragma unroll
-            for (int q4 = 0; q4 < kHistBins / 4; ++q4) {
-              const int4 v4 = __ldcg(gh + q4);
-              cnts[4 * q4] = v4.x; cnts[4 * q4 + 1] = v4.y; cnts[4 * q4 + 2] = v4.z; cnts[4 * q4 + 3] = v4.w;
-            }
-            int cum = 0, best = -1;
-#pragma unroll
-            for (int bb = kHistBins - 1; bb >= 1; --bb) {
-              cum += cnts[bb];
-              if (best < 0 && cum >= a.sel_count) best = bb;
-            }
-            if (best >= 1) {
-              // edge = thr0 + best * w; new emission threshold = edge - 2 eps
-              const float iw = multi ? __ldg(a.hist_inv_w + col) : s.inv_w[col];
-              if (iw > 0.f) {
-                const float nt = (multi ? __ldg(a.thr + col) : s.thr0[col]) + (float)best / iw - 2.f * a.eps[col];
-                if (nt > s.thr[col]) s.thr[col] = nt;
-              }
-            }
-          }
-        }
-        if (do_flush || periodic) epi_bar_sync();
-      }
-      if (++g == G0) g = 0;
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (PAIR) cluster_sync_all();   // the peer's smem / TMEM stay alive until the leader's last MMA has retired
-  if (warp == kMmaWarp) {
-    tc_fence_after();
-    if (PAIR) tmem_dealloc_2cta(tmem_base, (uint32_t)t.tmem_cols);
-    else tmem_dealloc(tmem_base, (uint32_t)t.tmem_cols);
-  }
-}
-
-// ---- DUAL: two corpus tiles per query slice ------------------------------------------------------------------
-// Measured (round 2, ncu + batch sweep): with the corpus in HBM, a step costs the HBM time of the corpus plus
-// ~0.055 ms per GB of QUERY image the SMs pull from L2 -- the image is re-streamed for every 128-row tile, 61 GB
-// per step at B = 256, as much as the corpus itself.  This variant lets a CTA hold TWO corpus tiles per K slice
-// and issue both MMAs (M = 128 each) against ONE copy of the query slice: the L2 -> SM query stream halves.
-// The two accumulators take all 512 TMEM columns, so the epilogue of a tile pair does not overlap the MMAs
-// of the next pair (the smem stages keep filling while it lasts).  One group of <= 256 queries per CTA
-// (B > 256 runs group-parallel lanes).
-//
-// Stage: [A tile 0 16 KB | A tile 1 16 KB | query slice nq * 128 B].  Same 14 warps as the single-tile kernel:
-// 0-3 epilogue (both tiles, one after the other; TMEM lane quarter = warp), 4 MMA issuer, 5 query producer,
-// 6-13 corpus loaders.  (Registers are allocated per 128 threads: a 576-thread block with four more epilogue
-// warps would be held to 96 registers per thread -- the probe in tools/probe_attrs.py shows it.)
-constexpr int kDualEpiWarps = kNumEpiWarps;
-constexpr int kDualMmaWarp = kMmaWarp;
-constexpr int kDualQWarp = kQWarp;
-constexpr int kDualFirstLoader = kFirstLoaderWarp;
-constexpr int kDualThreads = kThreads;   // 448
-__host__ __device__ inline uint32_t dual_stage_bytes(int nq) { return 2u * kABytes + (uint32_t)nq * 128u; }
-__device__ __forceinline__ void epi_bar_sync_dual() { epi_bar_sync(); }
-
-template <int METRIC, bool EF16>
-__global__ void __maxnreg__(128) scan_tcgen05_dual_kernel(const TcArgs t) {
-  extern __shared__ unsigned char smem_dyn[];
-  const int P = t.par_groups > 1 ? t.par_groups : 1;
-  const int pg = P > 1 ? (int)(blockIdx.x % (unsigned)P) : 0;
-  ScanArgs a = t.a;
-  const float* q_scale_g = t.q_scale;
-  const __half* qimg_g = t.qimg;
-  int nq = t.nq_last;                    // padded width of the group this CTA serves
-  if (P > 1) {
-    const int q0p = pg * kMaxQ;
-    a.B = min(kMaxQ, t.a.B - q0p);
-    a.thr += q0p; a.cand_cnt += q0p; a.eps += q0p; a.hist_inv_w += q0p; a.q_inv_norm += q0p;
-    if (a.cnt_all != nullptr) a.cnt_all += q0p;
-    a.dump += (size_t)q0p * a.n_sample_rows;
-    a.cand += (size_t)q0p * a.cap;
-    a.ghist += (size_t)q0p * kHistBins;
-    q_scale_g += q0p;
-    qimg_g += (size_t)pg * t.n_ks * kMaxQ * kSliceK;
-    nq = (pg == P - 1) ? t.nq_last : t.nq;
-  }
-  unsigned char* base = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
-  const uint32_t sbytes = dual_stage_bytes(t.nq);
-  SmemLayout s;
-  s.stage_base = base;
-  s.full = reinterpret_cast<uint64_t*>(base + (size_t)t.stages * sbytes);
-  s.empty = s.full + kMaxStages;
-  s.tmem_full = s.empty + kMaxStages;
-  s.tmem_empty = s.tmem_full + 2;
-  s.tmem_ptr = reinterpret_cast<uint32_t*>(s.tmem_empty + 2);
-  s.thr = reinterpret_cast<float*>(s.tmem_ptr + 4);
-  s.cs = s.thr + kMaxQ;
-  s.thr0 = s.cs + kMaxQ;
-  s.inv_w = s.thr0 + kMaxQ;
-  s.hist = reinterpret_cast<uint32_t*>(s.inv_w + kMaxQ);
-  s.cnt = reinterpret_cast<int*>(s.hist + kMaxQ * kHistBins / 2);
-  s.basev = s.cnt + kMaxQ;
-  s.list_n = s.basev + kMaxQ;
-  s.list = reinterpret_cast<uint32_t*>(s.list_n + 4);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // Work units: pairs of consecutive block ordinals (2u, 2u + 1); a missing second block is an empty tile.
-  const int64_t n_units = (a.n_mode_blocks + 1) / 2;
-  const int64_t first = (int64_t)blockIdx.x / P, stride = (int64_t)gridDim.x / P;
-  const int64_t my_units = first < n_units ? (n_units - first + stride - 1) / stride : 0;
-  auto ord_of = [&](int64_t unit, int half) -> int64_t { return 2 * (first + unit * stride) + half; };
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < t.stages; ++i) {
-      mbar_init(&s.full[i], 2 * kNumLoaderWarps + 1);   // 8 loader warps x 2 tiles + the query producer (expect_tx)
-      mbar_init(&s.empty[i], 1);                         // one tcgen05.commit
-    }
-    mbar_init(&s.tmem_full[0], 1);
-    mbar_init(&s.tmem_empty[0], kDualEpiWarps);
-    fence_barrier_init();
-  }
-  for (int i = threadIdx.x; i < kMaxQ; i += blockDim.x) {
-    s.thr[i] = (i < a.B && !a.dump_mode) ? a.thr[i] : __int_as_float(0x7f800000);  // +inf: never emit
-    s.cs[i] = (i < a.B) ? q_scale_g[i] : 0.f;
-    s.cnt[i] = 0;
-    s.thr0[i] = s.thr[i];
-    s.inv_w[i] = (i < a.B && !a.dump_mode) ? a.hist_inv_w[i] : 0.f;
-  }
-  for (int i = threadIdx.x; i < kMaxQ * kHistBins / 2; i += blockDim.x) s.hist[i] = 0u;
-  if (threadIdx.x == 0) { s.list_n[0] = 0; s.list_n[1] = 0; }
-  if (warp == kDualMmaWarp) tmem_alloc(s.tmem_ptr, 512u);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *s.tmem_ptr;
-  // (the launcher only picks this kernel when rows need no per-row scaling in the loader: cosine on a
-  // normalised corpus -- 1/|e| is applied in the epilogue -- or dot / l2 with their global power of two)
-  const int64_t total_items = my_units * t.n_ks * 2;   // loader items: (unit, K slice, tile half)
-
-  if (warp >= kDualFirstLoader) {
-    const int lt = threadIdx.x - kDualFirstLoader * 32;  // 0..255
-    const float gscale = (METRIC == RL_METRIC_COSINE) ? 1.f : pow2_scale(t.row_stats[1]);
-    const bool scale = !EF16 && gscale != 1.f;   // fp16-stored rows are used unscaled
-    // Per-thread geometry.  fp32 storage: float4 column c4 of rows r0 + 16 i (i < 8); fp16: 16-byte chunk j of
-    // rows r0 + 32 i (i < 4).  Both move 16 KB (one tile's K slice) per item.
-    const int c4 = lt & 15, r0f = lt >> 4;
-    const int j = lt & 7, r0h = lt >> 3;
-    const size_t esz = EF16 ? sizeof(__half) : sizeof(float);
-    const size_t slice_bytes = kSliceK * esz;
-    const size_t row_pitch = (size_t)a.ld * esz;
-    const unsigned char* Eb = reinterpret_cast<const unsigned char*>(a.E);
-    const uint32_t sw_f = (uint32_t)r0f * 128u + ((((uint32_t)c4 >> 1) ^ ((uint32_t)r0f & 7u)) << 4) + (((uint32_t)c4 & 1u) << 3);
-    const uint32_t sw_h = (uint32_t)r0h * 128u + (((uint32_t)j ^ ((uint32_t)r0h & 7u)) << 4);
-    // cursors: ld_* two items ahead of the stores, pf_* kPrefetchItems further ahead (L2 only)
-    struct Cur { int unit, ks, half, rows0, rows1; const unsigned char *p0, *p1; };
-    auto set_unit = [&](Cur& c, int thread_row, size_t col_bytes) {
-      c.rows0 = c.rows1 = 0;
-      if ((int64_t)c.unit < my_units) {
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-          const int64_t ord = ord_of((int64_t)c.unit, h);
-          if (ord < a.n_mode_blocks) {
-            const int64_t blk = mode_block_index(a, ord);
-            const int64_t rem = a.n_rows - blk * kTileM;
-            const int rows = rem < kTileM ? (int)rem : kTileM;
-            const unsigned char* p = Eb + (size_t)(blk * kTileM + thread_row) * row_pitch + col_bytes;
-            if (h == 0) { c.rows0 = rows; c.p0 = p; } else { c.rows1 = rows; c.p1 = p; }
-          }
-        }
-      }
-    };
-    auto advance = [&](Cur& c, int thread_row, size_t col_bytes) {
-      if (c.half == 0) c.p0 += slice_bytes; else c.p1 += slice_bytes;
-      c.half ^= 1;
-      if (c.half == 0 && ++c.ks == t.n_ks) { c.ks = 0; ++c.unit; set_unit(c, thread_row, col_bytes); }
-    };
-    Cur ld{0, 0, 0, 0, 0, nullptr, nullptr}, pf{0, 0, 0, 0, 0, nullptr, nullptr};
-    const int ld_row = EF16 ? r0h : r0f;
-    const size_t ld_col = EF16 ? (size_t)j * 16 : (size_t)c4 * 16;
-    const int pf_row = EF16 ? (lt & 127) : (lt >> 1);
-    const size_t pf_col = EF16 ? 0 : (size_t)(lt & 1) * 128;
-    auto prefetch_item = [&]() {   // one 128-byte line per thread (fp32: 2 lines per row slice, fp16: 1)
-      const int rows = pf.half ? pf.rows1 : pf.rows0;
-      const unsigned char* p = pf.half ? pf.p1 : pf.p0;
-      const bool active = EF16 ? lt < 128 : true;
-      if (pg == 0 && active && pf_row < rows && (size_t)pf.ks * slice_bytes + pf_col < (size_t)a.d * esz) prefetch_l2(p);
-      advance(pf, pf_row, pf_col);
-    };
-    uint4 ring[2][8];   // fp32: 8 x 16 B per item; fp16 uses the first 4
-    auto issue_item = [&](uint4 (&buf)[8]) {
-      const int rows = ld.half ? ld.rows1 : ld.rows0;
-      const unsigned char* p = ld.half ? ld.p1 : ld.p0;
-      const bool col_ok = (size_t)ld.ks * slice_bytes + ld_col < (size_t)a.d * esz;
-      if (EF16) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          buf[i] = (col_ok && r0h + 32 * i < rows) ? ldg_stream_u4(p) : make_uint4(0u, 0u, 0u, 0u);
-          p += 32 * row_pitch;
-        }
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          buf[i] = (col_ok && r0f + 16 * i < rows) ? ldg_stream_u4(p) : make_uint4(0u, 0u, 0u, 0u);
-          p += 16 * row_pitch;
-        }
-      }
-      advance(ld, ld_row, ld_col);
-      prefetch_item();
-    };
-    int stage = 0, st_half = 0;
-    uint32_t phase = 0;
-    const __half2 gs2 = __float2half2_rn(gscale);
-    auto process = [&](uint4 (&buf)[8]) {
-      mbar_wait(&s.empty[stage], phase ^ 1u);   // (second tile of a stage: same phase, passes at once)
-      unsigned char* A = s.stage_base + (size_t)stage * sbytes + (size_t)st_half * kABytes;
-      if (EF16) {
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          uint4 v = buf[i];
-          if (scale) {
-            __half2* h = reinterpret_cast<__half2*>(&v);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) h[e] = __hmul2(h[e], gs2);
-          }
-          *reinterpret_cast<uint4*>(A + sw_h + i * 32 * 128) = v;
-        }
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          const float4 f = *reinterpret_cast<const float4*>(&buf[i]);
-          const __half2 h01 = scale ? __floats2half2_rn(f.x * gscale, f.y * gscale) : __floats2half2_rn(f.x, f.y);
-          const __half2 h23 = scale ? __floats2half2_rn(f.z * gscale, f.w * gscale) : __floats2half2_rn(f.z, f.w);
-          uint2 packed;
-          packed.x = *reinterpret_cast<const uint32_t*>(&h01);
-          packed.y = *reinterpret_cast<const uint32_t*>(&h23);
-          *reinterpret_cast<uint2*>(A + sw_f + i * 16 * 128) = packed;
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&s.full[stage]);
-      issue_item(buf);
-      st_half ^= 1;
-      if (st_half == 0 && ++stage == t.stages) { stage = 0; phase ^= 1u; }
-    };
-    set_unit(ld, ld_row, ld_col);
-    set_unit(pf, pf_row, pf_col);
-    for (int i = 0; i < kPrefetchItems; ++i) prefetch_item();
-    issue_item(ring[0]);
-    issue_item(ring[1]);
-    for (int64_t item = 0; item < total_items; item += 2) {
-      process(ring[0]);
-      if (item + 1 < total_items) process(ring[1]);
-    }
-  } else if (warp == kDualQWarp) {
-    if (lane == 0) {
-      const uint32_t qbytes = (uint32_t)nq * 128u;   // one K slice of the group's queries
-      const unsigned char* qsrc = reinterpret_cast<const unsigned char*>(qimg_g);
-      const int64_t n_stages_total = my_units * t.n_ks;
-      int ks = 0, stage = 0;
-      uint32_t phase = 0;
-      for (int64_t it = 0; it < n_stages_total; ++it) {
-        mbar_wait(&s.empty[stage], phase ^ 1u);
-        mbar_arrive_expect_tx(&s.full[stage], qbytes);
-        bulk_g2s(s.stage_base + (size_t)stage * sbytes + 2 * kABytes, qsrc + (size_t)ks * qbytes, qbytes, &s.full[stage]);
-        if (++ks == t.n_ks) ks = 0;
-        if (++stage == t.stages) { stage = 0; phase ^= 1u; }
-      }
-    }
-  } else if (warp == kDualMmaWarp) {
-    if (lane == 0) {
-      const uint32_t idesc = make_idesc_f16(kTileM, nq);
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int64_t u = 0; u < my_units; ++u) {
-        mbar_wait(&s.tmem_empty[0], (uint32_t)((u & 1) ^ 1));   // both accumulators drained by the 8 epilogue warps
-        tc_fence_after();
-        const uint32_t d0 = tmem_base, d1 = tmem_base + (uint32_t)t.buf_cols;
-        for (int ks = 0; ks < t.n_ks; ++ks) {
-          mbar_wait(&s.full[stage], phase);
-          fence_proxy_async();
-          tc_fence_after();
-          const uint32_t a_addr = smem_u32(s.stage_base + (size_t)stage * sbytes);
-          const uint64_t a0 = make_kmajor_sw128_desc(a_addr), a1 = make_kmajor_sw128_desc(a_addr + kABytes);
-          const uint64_t b = make_kmajor_sw128_desc(a_addr + 2 * kABytes);
-#pragma unroll
-          for (int k = 0; k < kSliceK / 16; ++k) {
-            umma_f16(d0, a0 + (uint64_t)(2 * k), b + (uint64_t)(2 * k), idesc, (ks | k) != 0 ? 1u : 0u);
-            umma_f16(d1, a1 + (uint64_t)(2 * k), b + (uint64_t)(2 * k), idesc, (ks | k) != 0 ? 1u : 0u);
-          }
-          umma_commit(&s.empty[stage]);
-          if (++stage == t.stages) { stage = 0; phase ^= 1u; }
-        }
-        umma_commit(&s.tmem_full[0]);
-      }
-    }
-  } else {
-    // ===== epilogue warps 0..3 (TMEM lane quarter = warp): tile 0, then tile 1 of the pair =====
-    const int q = warp;
-    const bool cos_noscale = METRIC == RL_METRIC_COSINE;
-    bool flushed_once = false;
-    for (int64_t u = 0; u < my_units; ++u) {
-     mbar_wait(&s.tmem_full[0], (uint32_t)(u & 1));
-     tc_fence_after();
-     for (int half = 0; half < 2; ++half) {
-      const int64_t ord = ord_of(u, half);
-      const bool has_block = ord < a.n_mode_blocks;
-      const int64_t blk = has_block ? mode_block_index(a, ord) : 0;
-      const int r_in = q * 32 + lane;
-      const int64_t row = blk * kTileM + r_in;
-      bool valid = has_block && row < a.n_rows;
-      bool masked_alive = false;
-      if (valid && a.row_allowed != nullptr) {
-        valid = a.row_allowed[row] != 0;
-        if (!valid && a.cnt_all != nullptr) masked_alive = a.row_alive == nullptr || a.row_alive[row] != 0;
-      }
-      const float bias = (METRIC == RL_METRIC_L2 && valid) ? -a.sq_norm[row] : 0.f;
-      const float lane_scale = (cos_noscale && valid) ? __ldg(a.inv_norm + row) : 1.f;
-      const uint32_t taddr0 = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(half * t.buf_cols);
-      for (int c0 = 0; c0 < nq; c0 += 32) {
-        uint32_t v[32];
-        tmem_ld32_async(taddr0 + (uint32_t)c0, v);
-        tmem_ld_wait(v);
-        if (a.dump_mode) {
-#pragma unroll
-          for (int jj = 0; jj < 32; ++jj) {
-            const int col = c0 + jj;
-            if (col < a.B) {
-              float key = __uint_as_float(v[jj]);
-              if (METRIC != RL_METRIC_COSINE) key = fmaf(key, s.cs[col], bias);
-              else key *= lane_scale;
-              if (has_block) a.dump[(size_t)col * a.n_sample_rows + ord * kTileM + r_in] = valid ? key : kNegInf;
-            }
-          }
-        } else {
-          uint32_t mask = 0;
-#pragma unroll
-          for (int jj = 0; jj < 32; ++jj) {
-            float key = __uint_as_float(v[jj]);
-            if (METRIC != RL_METRIC_COSINE) key = fmaf(key, s.cs[c0 + jj], bias);
-            else key *= lane_scale;
-            if (key >= s.thr[c0 + jj]) mask |= 1u << jj;
-          }
-          if (masked_alive) {
-            uint32_t extra = mask;
-            while (extra != 0) {
-              const int jj = __ffs(extra) - 1;
-              extra &= extra - 1;
-              atomicAdd(a.cnt_all + c0 + jj, 1);
-            }
-          }
-          if (!valid) mask = 0;
-          while (mask != 0) {
-            const int jj = __ffs(mask) - 1;
-            mask &= mask - 1;
-            const int col = c0 + jj;
-            float key = __uint_as_float(select32(v, jj));
-            if (METRIC != RL_METRIC_COSINE) key = fmaf(key, s.cs[col], bias);
-            else key *= lane_scale;
-            const int pos = atomicAdd(&s.list_n[0], 1);
-            const int hb = col * kHistBins + hist_bin(key, s.thr0[col], s.inv_w[col]);
-            atomicAdd(&s.hist[hb >> 1], 1u << ((hb & 1) * 16));
-            if (pos < kListCap) {
-              s.list[pos * 3 + 0] = (uint32_t)col;
-              s.list[pos * 3 + 1] = __float_as_uint(key);
-              s.list[pos * 3 + 2] = (uint32_t)row;
-            } else {
-              emit_candidate(a, col, key, (int32_t)row);
-            }
-          }
-        }
-      }
-     }   // half
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&s.tmem_empty[0]);   // both accumulators are free once the 4 warps have arrived
-      if (!a.dump_mode) {
-        constexpr int NT = kDualEpiWarps * 32;
-        const int et = threadIdx.x;  // 0..255
-        epi_bar_sync_dual();
-        const int n_all = s.list_n[0];
-        epi_bar_sync_dual();
-        const bool last = u + 1 == my_units;
-        const bool do_flush = n_all >= (flushed_once ? kFlushAt : kFlushFirst) || (last && n_all > 0);
-        if (do_flush) {
-          flushed_once = true;
-          const int n = min(n_all, kListCap);
-          for (int e = et; e < n; e += NT) {
-            const int col = (int)s.list[e * 3 + 0];
-            s.list[e * 3 + 0] = (uint32_t)col | ((uint32_t)atomicAdd(&s.cnt[col], 1) << 16);
-          }
-          epi_bar_sync_dual();
-          for (int col = et; col < kMaxQ; col += NT) {
-            const int c = s.cnt[col];
-            if (c > 0) {
-              s.basev[col] = atomicAdd(a.cand_cnt + col, c);
-              s.cnt[col] = 0;
-            }
-          }
-          for (int w = et; w < kMaxQ * kHistBins / 2; w += NT) {
-            const uint32_t h = s.hist[w];
-            if (h != 0u) {
-              if (h & 0xFFFFu) atomicAdd(a.ghist + 2 * w, (int)(h & 0xFFFFu));
-              if (h >> 16) atomicAdd(a.ghist + 2 * w + 1, (int)(h >> 16));
-              s.hist[w] = 0u;
-            }
-          }
-          epi_bar_sync_dual();
-          if (et == 0) s.list_n[0] = 0;
-          for (int e = et; e < n; e += NT) {
-            const uint32_t w0 = s.list[e * 3 + 0];
-            const int col = (int)(w0 & 0xFFFFu);
-            const int slot = s.basev[col] + (int)(w0 >> 16);
-            if (slot < a.cap)
-              a.cand[(size_t)col * a.cap + slot] = Cand{__uint_as_float(s.list[e * 3 + 1]), (int32_t)s.list[e * 3 + 2]};
-          }
-        }
-        const bool periodic = (u % (kRefreshEvery / 2)) == kRefreshEvery / 2 - 1;   // a unit is two tiles
-        if ((do_flush || periodic) && !last) {
-          for (int col = et; col < a.B; col += NT) {
+          for (int col = et; col < a.B; col += kNumEpiWarps * 32) {
             const int4* gh = reinterpret_cast<const int4*>(a.ghist + (size_t)col * kHistBins);
             int cnts[kHistBins];
 #pragma unroll
@@ -1287,21 +822,24 @@ __global__ void __maxnreg__(128) scan_tcgen05_dual_kernel(const TcArgs t) {
               if (best < 0 && cum >= a.sel_count) best = bb;
             }
             if (best >= 1 && s.inv_w[col] > 0.f) {
+              // edge = thr0 + best * w; new emission threshold = edge - 2 eps
               const float nt = s.thr0[col] + (float)best / s.inv_w[col] - 2.f * a.eps[col];
               if (nt > s.thr[col]) s.thr[col] = nt;
             }
           }
         }
-        if (do_flush || periodic) epi_bar_sync_dual();
+        if (do_flush || periodic) epi_bar_sync();
       }
     }
   }
 
   tc_fence_before();
   __syncthreads();
-  if (warp == kDualMmaWarp) {
+  if (PAIR) cluster_sync_all();   // the peer's smem / TMEM stay alive until the leader's last MMA has retired
+  if (warp == kMmaWarp) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, 512u);
+    if (PAIR) tmem_dealloc_2cta(tmem_base, (uint32_t)t.tmem_cols);
+    else tmem_dealloc(tmem_base, (uint32_t)t.tmem_cols);
   }
 }
 
@@ -1396,30 +934,22 @@ static bool make_corpus_tensor_map(CUtensorMap* tm, const void* E, int64_t n_row
              CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-constexpr int kMaxGroups = 4;   // query groups walked per corpus tile in one launch (B <= 1024 per launch)
+constexpr int kMaxGroups = 4;   // query groups per launch (B <= 1024 per launch)
 
 int launch_scan_tcgen05(const ScanArgs& a_in, const rl_scan_params* p, const float* q_scale, const void* qimg,
                         int sm_count, cudaStream_t stream) {
   if (a_in.n_mode_blocks == 0 || a_in.B == 0) return RL_OK;
   const int n_ks = (p->d + kSliceK - 1) / kSliceK;
   const int groups = (a_in.B + kMaxQ - 1) / kMaxQ;
-  // Up to kMaxGroups groups of 256 queries share one launch so that HBM sees the corpus once (configs[2],
-  // B = 1024).  Two ways to share (RL_TC_GROUPMODE): "par" (default) -- the CTAs of a lane walk the same
-  // tiles at the same time, one group each, and meet in L2; "seq" -- every CTA walks its tiles once per
-  // group, back to back (measured: the 76 MB reuse distance defeats L2, HBM still reads the corpus 3.5x).
-  // RL_TC_GROUPS=1 restores one launch per group.
-  static const int max_groups = []() {
-    const char* e = getenv("RL_TC_GROUPS");
-    const int v = e ? atoi(e) : kMaxGroups;
-    return v < 1 ? 1 : (v > kMaxGroups ? kMaxGroups : v);
-  }();
-  static const bool seq_mode = []() { const char* e = getenv("RL_TC_GROUPMODE"); return e != nullptr && e[0] == 's'; }();
+  // The groups of 256 queries of one launch run group-parallel: the CTAs of a lane walk the same tiles at the
+  // same time, one group each, and meet in L2, so HBM sees the corpus once (configs[2], B = 1024).  A lane needs
+  // at least two SMs per group, which caps the groups per launch.
+  const int max_groups = min(kMaxGroups, max(1, sm_count / 2));
   // fp16 storage: the corpus tiles go HBM -> shared memory through a tensor map (TMA writes the swizzled UMMA tile,
-  // no loader warps, no registers in between).  RL_TC_TMA=0 keeps the register loaders (A/B).
+  // no loader warps, no registers in between); the register loaders take the corpora a tensor map cannot describe.
   CUtensorMap tmE;
   memset(&tmE, 0, sizeof(tmE));
-  static const bool tma_env = []() { const char* e = getenv("RL_TC_TMA"); return e == nullptr || atoi(e) != 0; }();
-  const bool tma_rows = p->e_dtype == 1 && tma_env && make_corpus_tensor_map(&tmE, p->E, p->n_rows, p->ld, p->d);
+  const bool tma_rows = p->e_dtype == 1 && make_corpus_tensor_map(&tmE, p->E, p->n_rows, p->ld, p->d);
   for (int g0 = 0; g0 < groups; g0 += max_groups) {
     TcArgs t;
     t.a = a_in;
@@ -1439,15 +969,11 @@ int launch_scan_tcgen05(const ScanArgs& a_in, const rl_scan_params* p, const flo
     t.qimg = reinterpret_cast<const __half*>(qimg) + (size_t)g0 * n_ks * kMaxQ * kSliceK;
     t.q_scale = q_scale + q0;
     t.row_stats = p->row_stats;
-    const bool par = ng > 1 && !seq_mode && sm_count >= 2 * ng;
-    t.n_groups = par ? 1 : ng;
-    t.par_groups = par ? ng : 1;
+    t.par_groups = ng;
     const int last_b = nb - (ng - 1) * kMaxQ;              // queries of the last group
     t.nq_last = (last_b + 15) / 16 * 16;
     t.nq = ng > 1 ? kMaxQ : t.nq_last;                     // a full group (the only group when ng == 1)
     t.n_ks = n_ks;
-    static const int pf_pairs_env = []() { const char* e = getenv("RL_TC_PF_PAIRS"); return e ? atoi(e) : kPrefetchItems / 2; }();
-    t.pf_pairs = pf_pairs_env < 0 ? 0 : (pf_pairs_env > 16 ? 16 : pf_pairs_env);
     t.tma_rows = tma_rows ? 1 : 0;
     t.buf_cols = (t.nq + 31) / 32 * 32;
     int cols = 32;
@@ -1455,24 +981,17 @@ int launch_scan_tcgen05(const ScanArgs& a_in, const rl_scan_params* p, const flo
     t.tmem_cols = cols;
     // cta_group::2 (SM pair): the two CTAs of a cluster issue ONE M = 256 MMA per K step and each holds only half
     // of the query slice, so an SM pulls 16 KB instead of 32 KB of query image per stage from L2 (the L2 -> SM
-    // stream: -25 % on an fp32 corpus, -33 % on fp16).  Default for a single query group (B <= 256) since the
-    // cluster-scope barrier operations left its hot loop: `mbarrier.arrive.release.cluster` compiles to
-    // MEMBAR.ALL.GPU + ERRBAR and `try_wait.acquire.cluster` to CCTL.IVALL, and the peer's per-stage relay
-    // thread paid that membar on every K slice -- 0.96 us per slice, the 15.4 ms this variant first measured
-    // against 12.4 ms for one CTA per SM.  With default-scope barrier operations (what CUTLASS's ClusterBarrier
-    // uses): 61 GB fp32 shard 11.87 vs 12.80 ms, fp16 shard 8.20 vs 8.67 ms, same box, back to back.  Group-parallel
-    // lanes (B > 256) do not gain (23.6 vs 23.1 ms: 74 clusters / 4 groups leave 4 SMs idle) and keep one CTA per
-    // SM unless RL_TC_PAIR=1 forces pairs; RL_TC_PAIR=0 turns them off everywhere.
-    static const int pair_env = []() { const char* e = getenv("RL_TC_PAIR"); return e ? atoi(e) : -1; }();
-    const bool pair_wanted = pair_env == 1 || (pair_env < 0 && ng == 1);
-    const bool pair = pair_wanted && t.nq % 32 == 0 && t.nq_last % 32 == 0 && t.nq_last >= 64 && a_in.n_mode_blocks >= 2 &&
+    // stream: -25 % on an fp32 corpus, -33 % on fp16).  Used for a single query group (B <= 256); the barrier
+    // operations in its hot loop are default-scope, since the cluster-scope ones compile to MEMBAR.ALL.GPU /
+    // CCTL.IVALL.  Group-parallel lanes (B > 256) do not gain from pairs and keep one CTA per SM (DESIGN.md 3.1).
+    const bool pair = ng == 1 && t.nq % 32 == 0 && t.nq_last % 32 == 0 && t.nq_last >= 64 && a_in.n_mode_blocks >= 2 &&
                       sm_count >= 2;
-    const uint32_t avail = kSmemBudget - 1024 - tail_bytes(t.n_groups);
+    const uint32_t avail = kSmemBudget - 1024 - tail_bytes();
     int stages = (int)(avail / stage_bytes(pair ? t.nq / 2 : t.nq));
     if (stages > kMaxStages) stages = kMaxStages;
     RL_REQUIRE(stages >= 2, RL_EUNSUPPORTED, "tcgen05 scan: not enough shared memory for 2 stages");
     t.stages = stages;
-    const size_t smem = (size_t)stages * stage_bytes(pair ? t.nq / 2 : t.nq) + tail_bytes(t.n_groups) + 1024;
+    const size_t smem = (size_t)stages * stage_bytes(pair ? t.nq / 2 : t.nq) + tail_bytes() + 1024;
     RL_REQUIRE(p->row_stats != nullptr, RL_EINVAL, "tcgen05 scan needs row_stats");
     auto launch = [&](auto kernel, bool is_pair) -> int {
       RL_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -1498,38 +1017,6 @@ int launch_scan_tcgen05(const ScanArgs& a_in, const rl_scan_params* p, const flo
     };
     int rc;
     const bool f16 = p->e_dtype == 1;
-    // Two corpus tiles per query slice (halves the L2 -> SM query stream): one query group per CTA, rows that
-    // need no per-row scaling in the loader.  Validated (the whole -m gpu suite passes with it) but measured
-    // SLOWER on B200 than the single-tile kernel, same box, back to back: 61 GB fp32 shard 14.1 vs 12.4 ms,
-    // fp16 shard 8.95 vs 8.81 ms, configs[2] 30.2 vs 21.6 ms -- with both accumulators live the epilogue no
-    // longer overlaps the next tile's MMAs and only three smem stages fit, which costs more than the halved
-    // query stream saves.  Opt-in: RL_TC_DUAL=1.
-    static const int dual_env = []() { const char* e = getenv("RL_TC_DUAL"); return e ? atoi(e) : 0; }();
-    const bool dual = dual_env == 1 && !pair && t.n_groups == 1 && a_in.n_mode_blocks >= 2 &&
-                      (p->metric != RL_METRIC_COSINE || p->rows_unit_scale == 1);
-    if (dual) {
-      const uint32_t avail_d = kSmemBudget - 1024 - tail_bytes(1);
-      int st = (int)(avail_d / dual_stage_bytes(t.nq));
-      if (st > kMaxStages) st = kMaxStages;
-      if (st >= 2) {
-        t.stages = st;
-        const size_t smem_d = (size_t)st * dual_stage_bytes(t.nq) + tail_bytes(1) + 1024;
-        auto launch_dual = [&](auto kernel) -> int {
-          RL_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_d));
-          const int64_t n_units = (a_in.n_mode_blocks + 1) / 2;
-          const int lanes = sm_count / t.par_groups;
-          const unsigned grid = (unsigned)((n_units < lanes ? n_units : lanes) * t.par_groups);
-          kernel<<<grid, kDualThreads, smem_d, stream>>>(t);
-          RL_CUDA_CHECK(cudaGetLastError());
-          return RL_OK;
-        };
-        if (p->metric == RL_METRIC_COSINE) rc = f16 ? launch_dual(scan_tcgen05_dual_kernel<RL_METRIC_COSINE, true>) : launch_dual(scan_tcgen05_dual_kernel<RL_METRIC_COSINE, false>);
-        else if (p->metric == RL_METRIC_DOT) rc = f16 ? launch_dual(scan_tcgen05_dual_kernel<RL_METRIC_DOT, true>) : launch_dual(scan_tcgen05_dual_kernel<RL_METRIC_DOT, false>);
-        else rc = f16 ? launch_dual(scan_tcgen05_dual_kernel<RL_METRIC_L2, true>) : launch_dual(scan_tcgen05_dual_kernel<RL_METRIC_L2, false>);
-        if (rc != RL_OK) return rc;
-        continue;
-      }
-    }
     auto dispatch = [&](auto metric_tag) -> int {
       constexpr int M = decltype(metric_tag)::value;
       if (pair) return f16 ? launch(scan_tcgen05_kernel<M, true, true>, true) : launch(scan_tcgen05_kernel<M, true, false>, true);
@@ -1541,30 +1028,6 @@ int launch_scan_tcgen05(const ScanArgs& a_in, const rl_scan_params* p, const flo
     if (rc != RL_OK) return rc;
   }
   return RL_OK;
-}
-
-// Debug probe: function attributes / occupancy of the scan kernels as the driver sees them.
-int debug_scan_kernel_attrs(int which, int* out) {
-  cudaFuncAttributes fa;
-  cudaError_t e = which == 0 ? cudaFuncGetAttributes(&fa, scan_tcgen05_kernel<0, false, false>)
-                             : (which == 1 ? cudaFuncGetAttributes(&fa, scan_tcgen05_dual_kernel<0, false>)
-                                           : cudaFuncGetAttributes(&fa, scan_tcgen05_dual_kernel<0, true>));
-  if (e != cudaSuccess) return (int)e;
-  out[0] = fa.numRegs; out[1] = fa.maxThreadsPerBlock; out[2] = (int)fa.sharedSizeBytes; out[3] = (int)fa.localSizeBytes;
-  out[4] = fa.maxDynamicSharedSizeBytes;
-  int nb = -1;
-  const size_t smem = 224448;
-  if (which >= 1) {
-    cudaFuncSetAttribute(which == 1 ? (const void*)scan_tcgen05_dual_kernel<0, false> : (const void*)scan_tcgen05_dual_kernel<0, true>,
-                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    e = which == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, scan_tcgen05_dual_kernel<0, false>, kDualThreads, smem)
-                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, scan_tcgen05_dual_kernel<0, true>, kDualThreads, smem);
-  }
-  out[5] = nb; out[6] = (int)e;
-  cudaDeviceProp prop;
-  cudaGetDeviceProperties(&prop, 0);
-  out[7] = prop.regsPerBlock; out[8] = prop.regsPerMultiprocessor; out[9] = (int)prop.sharedMemPerBlockOptin;
-  return 0;
 }
 
 }  // namespace rl

@@ -12,6 +12,4 @@ int tcgen05_prepare_queries(const rl_scan_params* p, const float* q_inv_norm, fl
 int launch_scan_tcgen05(const ScanArgs& a, const rl_scan_params* p, const float* q_scale, const void* qimg,
                         int sm_count, cudaStream_t stream);
 
-int debug_scan_kernel_attrs(int which, int* out);
-
 }  // namespace rl

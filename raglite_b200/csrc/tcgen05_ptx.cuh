@@ -208,22 +208,6 @@ __device__ __forceinline__ void umma_f16_2cta(uint32_t d_tmem, uint64_t a_desc, 
       : "memory");
 }
 
-// Bulk copy whose destination (and completing mbarrier) is the same shared-memory offset in every CTA of `mask`.
-__device__ __forceinline__ void bulk_g2s_multicast(void* smem_dst, const void* gsrc, uint32_t bytes, uint64_t* bar, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1], %2, [%3], %4;" ::"r"(
-          smem_u32(smem_dst)),
-      "l"(gsrc), "r"(bytes), "r"(smem_u32(bar)), "h"(mask)
-      : "memory");
-}
-// Commit of this CTA's (cta_group::1) MMAs that arrives on the barrier at the same offset in every CTA of `mask`.
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-
 __device__ __forceinline__ uint4 ldg_stream_u4(const void* p) {
   uint4 v;
   asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];"

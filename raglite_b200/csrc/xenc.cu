@@ -7,7 +7,7 @@
 //                        sliced by 64), X copied into 128B-swizzled smem by loader warps, W as a
 //                        pre-swizzled fp16 image fetched with cp.async.bulk, fp32 accumulate in TMEM,
 //                        bias / GELU(erf) fused in the TMEM epilogue
-//   attention_kernel     softmax(Q K^T / sqrt(dh)) V per (sequence, head), fp32 math
+//   attention2_kernel    softmax(Q K^T / sqrt(dh)) V per (sequence, head), fp32 math
 //   add_ln_kernel        LayerNorm(x + residual)
 //   cls_head_kernel      pooler (dense + tanh on [CLS]) -> classifier -> logit, sigmoid score
 #include <cuda.h>
@@ -117,7 +117,7 @@ struct LinArgs {
   __half* Y;           // [T, N]
   int T, N, K, act;    // act: 0 none, 1 GELU(erf)
   int n_pass, n_ks, stages;
-  int cp_async;        // 1: activation tile through cp.async (no register staging; every free stage in flight)
+  int cp_async;        // 1: activation tile through cp.async (launch_linear); 0: the register ring
   int pw;              // output columns per pass of the weight image (pass_width(N, K))
 };
 
@@ -132,12 +132,6 @@ __device__ __forceinline__ void cp_async_mbar_arrive_noinc(uint64_t* bar) {
 
 __host__ __device__ inline uint32_t lin_stage_bytes() { return kABytes + kMaxN * 128u; }
 
-// MC: a cluster of two CTAs works on two token tiles of the SAME output pass; every weight slice is fetched from
-// L2 once per cluster -- CTA r issues half r with .multicast::cluster, it lands at the same offset in both CTAs --
-// so the L2 -> SM weight stream, which bounds the K = 1536 layer (FFN-down: 590 KB of weights per 128-token
-// tile, 788 MB per launch at ~8.7 TB/s), halves.  A stage is refilled only when BOTH CTAs' MMAs have released
-// it: the commit that frees a stage is multicast to both CTAs' empty barriers (count 2).
-template <bool MC>
 __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinArgs t) {
   extern __shared__ unsigned char smem_dyn[];
   unsigned char* base = smem_dyn + ((1024u - (smem_u32(smem_dyn) & 1023u)) & 1023u);
@@ -151,18 +145,16 @@ __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinAr
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int m_tiles = (t.T + kTileM - 1) / kTileM;
-  // item = m_unit * n_pass + pass; a unit is one token tile, or (MC) the pair of tiles 2u, 2u + 1 of a cluster
-  const uint32_t crank = MC ? cluster_ctarank() : 0u;
-  const int m_units = MC ? (m_tiles + 1) / 2 : m_tiles;
-  const int64_t n_items = (int64_t)m_units * t.n_pass;
-  const int64_t first = MC ? blockIdx.x >> 1 : blockIdx.x, stride = MC ? gridDim.x >> 1 : gridDim.x;
+  // item = m_tile * n_pass + pass
+  const int64_t n_items = (int64_t)m_tiles * t.n_pass;
+  const int64_t first = blockIdx.x, stride = gridDim.x;
   const int64_t my_items = first < n_items ? (n_items - first + stride - 1) / stride : 0;
-  auto tile_of = [&](int64_t item) -> int { const int u = (int)(item / t.n_pass); return MC ? 2 * u + (int)crank : u; };
+  auto tile_of = [&](int64_t item) -> int { return (int)(item / t.n_pass); };
 
   if (threadIdx.x == 0) {
     for (int i = 0; i < t.stages; ++i) {
       mbar_init(&full[i], (t.cp_async ? kNumLoaderWarps * 32 : kNumLoaderWarps) + 1);
-      mbar_init(&empty[i], MC ? 2 : 1);
+      mbar_init(&empty[i], 1);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tmem_full[i], 1);
@@ -173,7 +165,6 @@ __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinAr
   if (warp == kMmaWarp) tmem_alloc(tmem_ptr, 512);
   tc_fence_before();
   __syncthreads();
-  if (MC) cluster_sync_all();   // the peer's barriers are initialised before any multicast / remote commit reaches them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
 
@@ -213,9 +204,9 @@ __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinAr
       if (++stage == t.stages) { stage = 0; phase ^= 1u; }
     };
     if (t.cp_async) {
-      // Experimental (RL_XENC_CPASYNC=1): each thread fires its four 16-byte copies straight into the
-      // swizzled tile and lets the hardware arrive on the stage's barrier when they land, so the
-      // loaders run ahead by as many stages as are free instead of by the depth of a register ring.
+      // Each thread fires its four 16-byte copies straight into the swizzled tile and lets the hardware arrive on
+      // the stage's barrier when they land, so the loaders run ahead by as many stages as are free instead of by
+      // the depth of a register ring (352 vs 309 us for a layer's four GEMMs, profiles/r01_linear_loader_ab.json).
       for (int64_t g = 0; g < n_slices; ++g) {
         const int64_t it = g / t.n_ks;
         const int ks = (int)(g - it * t.n_ks);
@@ -261,14 +252,7 @@ __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinAr
         for (int ks = 0; ks < t.n_ks; ++ks) {
           mbar_wait(&empty[stage], phase ^ 1u);
           mbar_arrive_expect_tx(&full[stage], wbytes);
-          if (MC) {   // this CTA's half of the slice, to both CTAs of the cluster
-            const uint32_t half = wbytes / 2;
-            bulk_g2s_multicast(base + (size_t)stage * sbytes + kABytes + (size_t)crank * half,
-                               reinterpret_cast<const unsigned char*>(src + (size_t)ks * nb * kSliceK) + (size_t)crank * half, half,
-                               &full[stage], (uint16_t)3);
-          } else {
-            bulk_g2s(base + (size_t)stage * sbytes + kABytes, src + (size_t)ks * nb * kSliceK, wbytes, &full[stage]);
-          }
+          bulk_g2s(base + (size_t)stage * sbytes + kABytes, src + (size_t)ks * nb * kSliceK, wbytes, &full[stage]);
           if (++stage == t.stages) { stage = 0; phase ^= 1u; }
         }
       }
@@ -296,8 +280,7 @@ __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinAr
 #pragma unroll
           for (int k = 0; k < kSliceK / 16; ++k)
             umma_f16(d_tmem, a_desc + (uint64_t)(2 * k), b_desc + (uint64_t)(2 * k), idesc, (ks | k) != 0 ? 1u : 0u);
-          if (MC) umma_commit_mc(&empty[stage], (uint16_t)3);   // frees the stage in both CTAs (count 2)
-          else umma_commit(&empty[stage]);
+          umma_commit(&empty[stage]);
           if (++stage == t.stages) { stage = 0; phase ^= 1u; }
         }
         umma_commit(&tmem_full[buf]);
@@ -360,7 +343,6 @@ __global__ void __launch_bounds__(kThreads, 1) linear_tcgen05_kernel(const LinAr
   }
   tc_fence_before();
   __syncthreads();
-  if (MC) cluster_sync_all();   // no CTA leaves while its peer may still multicast into it or commit to its barriers
   if (warp == kMmaWarp) {
     tc_fence_after();
     tmem_dealloc(tmem_base, 512);
@@ -682,192 +664,6 @@ __device__ __forceinline__ float ex2_approx(float x) {   // 2^x, one MUFU op; ex
   return y;
 }
 
-// 4 x 4 transpose of 32-bit words across the four lanes of a quad: afterwards w[l] on lane c holds what
-// w[c] was on lane l.  Turns "16 contiguous bytes of a row per lane" (one 64-byte request per row) into
-// the m16n8k16 fragment layout (4-byte pieces at stride 16 bytes) and back.
-__device__ __forceinline__ void quad_transpose(uint32_t (&w)[4], int c) {
-#pragma unroll
-  for (int s = 1; s < 4; ++s) {   // selects only: a branch here would make the shuffle divergent
-    const int p = c ^ s;
-    const uint32_t lo = (p & 1) ? w[1] : w[0], hi = (p & 1) ? w[3] : w[2];
-    const uint32_t got = __shfl_xor_sync(0xffffffffu, (p & 2) ? hi : lo, s);
-    w[0] = p == 0 ? got : w[0];
-    w[1] = p == 1 ? got : w[1];
-    w[2] = p == 2 ? got : w[2];
-    w[3] = p == 3 ? got : w[3];
-  }
-}
-
-template <bool QUAD>   // QUAD: 16-byte Q loads / context stores through a quad transpose; else (default) 4-byte fragment pieces
-__global__ void __launch_bounds__(128, 5) attention_kernel(const __half* __restrict__ qkv, const int32_t* __restrict__ cu,
-                                                        int H, int n_heads, float scale_log2e, __half* __restrict__ ctx,
-                                                        int len_lo, int len_hi) {
-  extern __shared__ __align__(16) unsigned char att_smem[];
-  const int seq = blockIdx.x, head = blockIdx.y;
-  const int t0 = cu[seq], L = cu[seq + 1] - t0;
-  // Length buckets: the launch's shared memory is sized for len_hi keys, so a launch for the short sequences
-  // keeps five CTAs per SM resident (41 KB each at 256 keys) instead of the three a 512-key allocation allows.
-  if (L <= len_lo || L > len_hi) return;
-  const int Lp = (L + 63) / 64 * 64;
-  __half* Ks = reinterpret_cast<__half*>(att_smem);
-  __half* Vs = Ks + (size_t)Lp * kAttPitch;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const size_t ld = (size_t)3 * H;
-#pragma unroll 4
-  for (int idx = threadIdx.x; idx < Lp * 4; idx += blockDim.x) {
-    const int j = idx >> 2, c = idx & 3;
-    uint4 kv = make_uint4(0u, 0u, 0u, 0u), vv = kv;
-    if (j < L) {
-      const __half* base = qkv + (size_t)(t0 + j) * ld + head * 32 + c * 8;
-      kv = __ldg(reinterpret_cast<const uint4*>(base + H));
-      vv = __ldg(reinterpret_cast<const uint4*>(base + 2 * H));
-    }
-    *reinterpret_cast<uint4*>(Ks + (size_t)j * kAttPitch + c * 8) = kv;
-    *reinterpret_cast<uint4*>(Vs + (size_t)j * kAttPitch + c * 8) = vv;
-  }
-  __syncthreads();
-  const int r = lane >> 2, cp = (lane & 3) * 2;
-  // Q fragments (A operand of S = Q K^T) of a 16-query block; the next block's are fetched while this
-  // one is computed.
-  const int qc = lane & 3;
-  auto load_q = [&](int qb, uint32_t (&a)[2][4]) {   // raw 16-byte row chunks; finish_q turns them into fragments
-    const int q0 = qb * 16 + r, q1 = q0 + 8;
-    if (!QUAD) {
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks) {
-        const __half* p0 = qkv + (size_t)(t0 + q0) * ld + head * 32 + ks * 16 + cp;
-        const __half* p1 = qkv + (size_t)(t0 + q1) * ld + head * 32 + ks * 16 + cp;
-        a[ks][0] = q0 < L ? __ldg(reinterpret_cast<const uint32_t*>(p0)) : 0u;
-        a[ks][1] = q1 < L ? __ldg(reinterpret_cast<const uint32_t*>(p1)) : 0u;
-        a[ks][2] = q0 < L ? __ldg(reinterpret_cast<const uint32_t*>(p0 + 8)) : 0u;
-        a[ks][3] = q1 < L ? __ldg(reinterpret_cast<const uint32_t*>(p1 + 8)) : 0u;
-      }
-      return;
-    }
-    const uint4 z = make_uint4(0u, 0u, 0u, 0u);
-    const uint4 u0 = q0 < L ? __ldg(reinterpret_cast<const uint4*>(qkv + (size_t)(t0 + q0) * ld + head * 32 + qc * 8)) : z;
-    const uint4 u1 = q1 < L ? __ldg(reinterpret_cast<const uint4*>(qkv + (size_t)(t0 + q1) * ld + head * 32 + qc * 8)) : z;
-    a[0][0] = u0.x; a[0][1] = u0.y; a[0][2] = u0.z; a[0][3] = u0.w;
-    a[1][0] = u1.x; a[1][1] = u1.y; a[1][2] = u1.z; a[1][3] = u1.w;
-  };
-  auto finish_q = [&](const uint32_t (&raw)[2][4], uint32_t (&a)[2][4]) {
-    if (!QUAD) {
-#pragma unroll
-      for (int ks = 0; ks < 2; ++ks)
-#pragma unroll
-        for (int e = 0; e < 4; ++e) a[ks][e] = raw[ks][e];
-      return;
-    }
-    uint32_t w0[4] = {raw[0][0], raw[0][1], raw[0][2], raw[0][3]};
-    uint32_t w1[4] = {raw[1][0], raw[1][1], raw[1][2], raw[1][3]};
-    quad_transpose(w0, qc);   // w0[l] = row q0, columns l*8 + cp, +1
-    quad_transpose(w1, qc);
-    a[0][0] = w0[0]; a[0][2] = w0[1]; a[1][0] = w0[2]; a[1][2] = w0[3];
-    a[0][1] = w1[0]; a[0][3] = w1[1]; a[1][1] = w1[2]; a[1][3] = w1[3];
-  };
-  uint32_t a[2][4], a_next[2][4];
-  load_q(warp, a_next);   // rows >= L read as zero, so a block past the end is harmless
-  for (int qb = warp; qb * 16 < L; qb += 4) {
-    const int q0 = qb * 16 + r, q1 = q0 + 8;
-    finish_q(a_next, a);
-    load_q(qb + 4, a_next);
-    float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;
-    float O[4][4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-      for (int e = 0; e < 4; ++e) O[i][e] = 0.f;
-    for (int kb = 0; kb < Lp; kb += 64) {
-      float S[8][4];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-#pragma unroll
-        for (int e = 0; e < 4; ++e) S[j][e] = 0.f;
-        uint32_t b[4];
-        ldsm_x4(b, Ks + (size_t)(kb + j * 8 + (lane & 7)) * kAttPitch + (lane >> 3) * 8);
-        mma16816(S[j], a[0], b[0], b[1]);
-        mma16816(S[j], a[1], b[2], b[3]);
-      }
-      // Online softmax in the exp2 domain.  The running maxima are kept scaled (m = max(S) * scale);
-      // the scale itself is folded into the exponent's FMA, so a score costs one FMNMX, one FFMA, one
-      // ex2 and one FADD.  Only the last key block holds padding keys.
-      float mx0 = -INFINITY, mx1 = -INFINITY;
-      if (kb + 64 > L) {
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-#pragma unroll
-          for (int e = 0; e < 4; ++e)
-            if (kb + j * 8 + cp + (e & 1) >= L) S[j][e] = -INFINITY;
-      }
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        mx0 = fmaxf(mx0, fmaxf(S[j][0], S[j][1]));
-        mx1 = fmaxf(mx1, fmaxf(S[j][2], S[j][3]));
-      }
-      mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
-      mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
-      mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
-      mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
-      // finite: every key block holds a valid key (scale > 0, so max commutes with the scaling)
-      const float mn0 = fmaxf(m0, mx0 * scale_log2e), mn1 = fmaxf(m1, mx1 * scale_log2e);
-      const float c0 = ex2_approx(m0 - mn0), c1 = ex2_approx(m1 - mn1);
-      l0 *= c0; l1 *= c1;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) { O[i][0] *= c0; O[i][1] *= c0; O[i][2] *= c1; O[i][3] *= c1; }
-#pragma unroll
-      for (int j = 0; j < 8; ++j)
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const float pexp = ex2_approx(fmaf(S[j][e], scale_log2e, e < 2 ? -mn0 : -mn1));   // -inf -> 0
-          S[j][e] = pexp;
-          if (e < 2) l0 += pexp; else l1 += pexp;
-        }
-      m0 = mn0; m1 = mn1;
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) {
-        uint32_t pa[4];
-        pa[0] = pack_half2(S[2 * kk][0], S[2 * kk][1]);
-        pa[1] = pack_half2(S[2 * kk][2], S[2 * kk][3]);
-        pa[2] = pack_half2(S[2 * kk + 1][0], S[2 * kk + 1][1]);
-        pa[3] = pack_half2(S[2 * kk + 1][2], S[2 * kk + 1][3]);
-#pragma unroll
-        for (int dn2 = 0; dn2 < 2; ++dn2) {
-          uint32_t vb[4];
-          ldsm_x4_trans(vb, Vs + (size_t)(kb + kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8) * kAttPitch +
-                                (dn2 * 2 + (lane >> 4)) * 8);
-          mma16816(O[dn2 * 2], pa, vb[0], vb[1]);
-          mma16816(O[dn2 * 2 + 1], pa, vb[2], vb[3]);
-        }
-      }
-    }
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 1);
-    l0 += __shfl_xor_sync(0xffffffffu, l0, 2);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 1);
-    l1 += __shfl_xor_sync(0xffffffffu, l1, 2);
-    const float inv0 = 1.f / l0, inv1 = 1.f / l1;
-    uint32_t o0[4], o1[4];
-#pragma unroll
-    for (int dn = 0; dn < 4; ++dn) {
-      o0[dn] = pack_half2(O[dn][0] * inv0, O[dn][1] * inv0);
-      o1[dn] = pack_half2(O[dn][2] * inv1, O[dn][3] * inv1);
-    }
-    if (!QUAD) {
-#pragma unroll
-      for (int dn = 0; dn < 4; ++dn) {
-        if (q0 < L) *reinterpret_cast<uint32_t*>(ctx + (size_t)(t0 + q0) * H + head * 32 + dn * 8 + cp) = o0[dn];
-        if (q1 < L) *reinterpret_cast<uint32_t*>(ctx + (size_t)(t0 + q1) * H + head * 32 + dn * 8 + cp) = o1[dn];
-      }
-      continue;
-    }
-    quad_transpose(o0, qc);   // lane qc now holds columns qc*8 .. qc*8+7 of its rows: one 16-byte store each
-    quad_transpose(o1, qc);
-    if (q0 < L)
-      *reinterpret_cast<uint4*>(ctx + (size_t)(t0 + q0) * H + head * 32 + qc * 8) = make_uint4(o0[0], o0[1], o0[2], o0[3]);
-    if (q1 < L)
-      *reinterpret_cast<uint4*>(ctx + (size_t)(t0 + q1) * H + head * 32 + qc * 8) = make_uint4(o1[0], o1[1], o1[2], o1[3]);
-  }
-}
-
 // Sequence indices of a call sorted by length, longest first (counting sort over the lengths; equal lengths in any
 // order).  One CTA, once per forward.
 constexpr int kMaxSeqLenBins = 2048;
@@ -898,8 +694,9 @@ __global__ void __launch_bounds__(128, 3) attention2_kernel(const __half* __rest
                                                          const int32_t* __restrict__ order, int H, int n_heads,
                                                          float scale_log2e, __half* __restrict__ ctx, int n_seq, int seq_fastest, int stage_async) {
   extern __shared__ __align__(16) unsigned char att_smem[];
-  // CTA -> (sequence slot, head): heads fastest (the twelve CTAs of a sequence run together and read the same qkv
-  // rows), or sequences fastest (RL_XENC_ATT_ORDER=1, the A/B alternative: every head walks the length-sorted list).
+  // CTA -> (sequence slot, head): heads fastest (the twelve CTAs of a sequence run together and read the same qkv rows).
+  // The run-time seq_fastest / stage_async / null-order cases are what rl_xenc_score does not use; folding them away
+  // costs this kernel 52 bytes of spills at its 168-register cap (three CTAs per SM), so they stay parameters.
   const int head = seq_fastest ? (int)(blockIdx.x / (unsigned)n_seq) : (int)(blockIdx.x % (unsigned)n_heads);
   const int slot = seq_fastest ? (int)(blockIdx.x % (unsigned)n_seq) : (int)(blockIdx.x / (unsigned)n_heads);
   const int seq = order != nullptr ? order[slot] : slot;
@@ -1205,51 +1002,25 @@ static int launch_linear_resident(const __half* X, const void* img, const float*
 
 static int launch_linear(const __half* X, const void* img, const float* bias, __half* Y, int T, int N, int K, int act,
                          int sm_count, cudaStream_t stream) {
-  // RL_XENC_RESIDENT=0 forces the streaming kernel (A/B switch; the image layout follows pass_width()).
-  const char* res_env = getenv("RL_XENC_RESIDENT");   // read per launch: tools/time_linear.py A/Bs it in one process
-  const bool resident_ok = res_env == nullptr || atoi(res_env) != 0;
-  if (use_resident(N, K)) {
-    if (resident_ok) return launch_linear_resident(X, img, bias, Y, T, N, K, act, sm_count, stream);
-  }
+  if (use_resident(N, K)) return launch_linear_resident(X, img, bias, Y, T, N, K, act, sm_count, stream);
   LinArgs t;
   t.X = X; t.img = reinterpret_cast<const __half*>(img); t.bias = bias; t.Y = Y; t.T = T; t.N = N; t.K = K; t.act = act;
   t.pw = pass_width(N, K);
   t.n_pass = (N + t.pw - 1) / t.pw;
   t.n_ks = (K + kSliceK - 1) / kSliceK;
-  // cp.async activation loader (every free smem stage in flight, no registers held) is the default: bit-identical
-  // outputs, 352 -> 309 us for the four GEMMs of a layer (profiles/r01_linear_loader_ab.json); RL_XENC_CPASYNC=0
-  // selects the register-ring loader.  Read per launch: tools/time_linear.py A/Bs it in one process.
-  const char* cpa = getenv("RL_XENC_CPASYNC");
-  t.cp_async = (cpa != nullptr && atoi(cpa) == 0) ? 0 : 1;
+  // The cp.async loader is the one used.  The register-ring branch stays in the kernel because the kernel with it
+  // folded away measured slower on B200 (FFN-down, K = 1536: 95.5 vs 92.5 us, tools/time_linear.py).
+  t.cp_async = 1;
   static_assert((2 * kMaxStages + 4) * 8 + 8 <= kBarBytes, "barrier block overflows its slot");
   const uint32_t tail = kBarBytes + kEpiBytes;
   int stages = (int)((kSmemBudget - 1024 - tail) / lin_stage_bytes());
   if (stages > kMaxStages) stages = kMaxStages;
   t.stages = stages;
   const size_t smem = (size_t)stages * lin_stage_bytes() + tail + 1024;
-  // Cluster multicast of the weight slices (two token tiles per cluster).  Validated bit-identical, measured no
-  // gain on B200 (FFN-down 89.9 us vs 88.6 us without, tools/time_linear.py): at cluster size 2 L2 already merges
-  // the two CTAs' unicast requests for the same lines, so the multicast removes no traffic.  Opt-in: RL_XENC_MC=1.
-  const char* mc_env = getenv("RL_XENC_MC");
-  const bool mc = (mc_env != nullptr && atoi(mc_env) != 0) && t.cp_async && T > kTileM && sm_count >= 2 &&
-                  (((N + t.pw - 1) / t.pw == N / t.pw) && (t.pw * 128) % 32 == 0);
-  if (mc) {
-    RL_CUDA_CHECK(cudaFuncSetAttribute(linear_tcgen05_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int64_t units = (int64_t)(((T + kTileM - 1) / kTileM + 1) / 2) * t.n_pass;
-    const int clusters = (int)(units < sm_count / 2 ? units : sm_count / 2);
-    cudaLaunchConfig_t cfg{};
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.gridDim = dim3((unsigned)(2 * clusters)); cfg.blockDim = dim3(kThreads); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    RL_CUDA_CHECK(cudaLaunchKernelEx(&cfg, linear_tcgen05_kernel<true>, t));
-    return RL_OK;
-  }
-  RL_CUDA_CHECK(cudaFuncSetAttribute(linear_tcgen05_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  RL_CUDA_CHECK(cudaFuncSetAttribute(linear_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int64_t items = (int64_t)((T + kTileM - 1) / kTileM) * t.n_pass;
   const int grid = (int)(items < sm_count ? items : sm_count);
-  linear_tcgen05_kernel<false><<<grid, kThreads, smem, stream>>>(t);
+  linear_tcgen05_kernel<<<grid, kThreads, smem, stream>>>(t);
   RL_CUDA_CHECK(cudaGetLastError());
   return RL_OK;
 }
@@ -1298,15 +1069,9 @@ extern "C" int rl_xenc_score(const rl_xenc_weights* w, const int32_t* input_ids,
   int32_t* seq_order = reinterpret_cast<int32_t*>(
       (reinterpret_cast<uintptr_t>(ffn + (size_t)T * F) + 15) & ~uintptr_t(15));   // [P] (P <= T)
   RL_REQUIRE(P <= T, RL_EINVAL, "rl_xenc_score: more sequences than tokens");
-  // Attention walks the sequences longest first (RL_XENC_ATT_LPT=0: in arrival order, the A/B baseline).
-  static const bool att_lpt = []() { const char* e = getenv("RL_XENC_ATT_LPT"); return e == nullptr || atoi(e) != 0; }();
-  // K / V staging through cp.async with the first Q loads overlapped (RL_XENC_ATT_CPASYNC=0: plain loads, the A/B baseline)
-  static const bool att_stage_async = []() { const char* e = getenv("RL_XENC_ATT_CPASYNC"); return e == nullptr || atoi(e) != 0; }();
-  static const bool att_seq_fastest = []() { const char* e = getenv("RL_XENC_ATT_ORDER"); return e != nullptr && atoi(e) == 1; }();
-  if (att_lpt) {
-    seq_order_kernel<<<1, 1024, 0, stream>>>(cu_seqlens, P, seq_order);
-    RL_CUDA_CHECK(cudaGetLastError());
-  }
+  // Attention walks the sequences longest first.
+  seq_order_kernel<<<1, 1024, 0, stream>>>(cu_seqlens, P, seq_order);
+  RL_CUDA_CHECK(cudaGetLastError());
   const int tok_blocks = (T + 7) / 8;
   const bool ln_vec = H % 128 == 0;   // (LayerNorm gamma / beta come from torch allocations: 16-byte aligned)
   embed_ln_kernel<<<tok_blocks, 256, 0, stream>>>(input_ids, type_ids, pos_ids, reinterpret_cast<const __half*>(w->word_emb),
@@ -1316,40 +1081,14 @@ extern "C" int rl_xenc_score(const rl_xenc_weights* w, const int32_t* input_ids,
   RL_CUDA_CHECK(cudaGetLastError());
   const size_t att_smem = (size_t)((max_len + 63) / 64 * 64) * kAttPitch * 2 * sizeof(__half);
   RL_REQUIRE(att_smem <= 200 * 1024, RL_EUNSUPPORTED, "rl_xenc_score: max_len=%d too long for the attention kernel", max_len);
-  // Two launches when the batch holds long sequences: keys <= kAttShort with a small allocation (occupancy), the rest
-  // with the full one.  (ncu, round 2: a single launch sized by the longest sequence ran 3 CTAs = 12 warps per SM.)
-  constexpr int kAttShort = 256;
-  const size_t att_smem_short = (size_t)kAttShort * kAttPitch * 2 * sizeof(__half);
-  // A/B switch for the Q loads / context stores.  Measured back to back on one B200 (262 k tokens per
-  // layer): 4-byte fragment pieces 0.744 ms, 16-byte rows + quad transpose 1.100 ms -- so pieces are
-  // the default and RL_XENC_ATT_QUAD=1 selects the transpose variant.
-  static const bool att_quad = []() { const char* e = getenv("RL_XENC_ATT_QUAD"); return e ? atoi(e) != 0 : false; }();
-  RL_CUDA_CHECK(cudaFuncSetAttribute(attention_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem));
-  RL_CUDA_CHECK(cudaFuncSetAttribute(attention_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem));
   RL_CUDA_CHECK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem));
   const float scale = 1.4426950408889634f / sqrtf(32.f);  // softmax in the exp2 domain
   for (int l = 0; l < w->n_layers; ++l) {
     const rl_xenc_layer& L = w->layers[l];
     int rc = launch_linear(hidden, L.qkv_img, L.qkv_bias, qkv, T, 3 * H, H, 0, sms, stream);
     if (rc != RL_OK) return rc;
-    static const bool att2 = []() { const char* e = getenv("RL_XENC_ATT2"); return e == nullptr || atoi(e) != 0; }();
-    auto attention = [&](size_t smem, int lo, int hi) {
-      if (att2 && lo == 0 && hi == max_len)
-        attention2_kernel<<<dim3((unsigned)P * (unsigned)nh), 128, smem, stream>>>(qkv, cu_seqlens, att_lpt ? seq_order : nullptr, H, nh, scale, ctx,
-                                                                                       P, att_seq_fastest ? 1 : 0, att_stage_async ? 1 : 0);
-      else if (att_quad) attention_kernel<true><<<dim3(P, nh), 128, smem, stream>>>(qkv, cu_seqlens, H, nh, scale, ctx, lo, hi);
-      else attention_kernel<false><<<dim3(P, nh), 128, smem, stream>>>(qkv, cu_seqlens, H, nh, scale, ctx, lo, hi);
-    };
-    // Measured (ncu launch list, 51 k tokens per call, mean 200): two bucketed launches 86 + 64 us vs 141 us for one
-    // launch -- the long sequences carry 40 % of the L^2 work and gain nothing, the split adds a tail.  Off
-    // unless RL_XENC_ATT_BUCKETS=1.
-    static const bool buckets = []() { const char* e = getenv("RL_XENC_ATT_BUCKETS"); return e != nullptr && atoi(e) != 0; }();
-    if (buckets && max_len > kAttShort) {
-      attention(att_smem_short, 0, kAttShort);
-      attention(att_smem, kAttShort, max_len);
-    } else {
-      attention(att_smem, 0, max_len);
-    }
+    attention2_kernel<<<(unsigned)P * (unsigned)nh, 128, att_smem, stream>>>(qkv, cu_seqlens, seq_order, H, nh, scale, ctx,
+                                                                            P, /*seq_fastest=*/0, /*stage_async=*/1);
     RL_CUDA_CHECK(cudaGetLastError());
     rc = launch_linear(ctx, L.o_img, L.o_bias, tmp, T, H, H, 0, sms, stream);
     if (rc != RL_OK) return rc;

@@ -1,8 +1,7 @@
-"""A/B of the cross-encoder linear kernels: weight-resident + TMA tensor-map loader (default for K <= 384),
-streaming kernel with the cp.async loader, streaming kernel with the register-ring loader.  Parity of every
-GEMM shape against torch (incl. a ragged token count), then CUDA-event timing of back-to-back launches."""
+"""Cross-encoder linear layer as rl_xenc_linear dispatches it (weight-resident kernel for K <= 384, streaming
+kernel otherwise): parity of every GEMM shape against torch (incl. a ragged token count), then CUDA-event timing
+of back-to-back launches."""
 import json
-import os
 import sys
 from pathlib import Path
 
@@ -28,24 +27,20 @@ for name, N, K, act in shapes:
     if act:
         ref = torch.nn.functional.gelu(ref)
     Y = torch.empty((T, N), dtype=torch.float16, device="cuda")
-    for mode, (res, cpa, mc) in {"resident": ("1", "1", "0"), "stream_multicast": ("0", "1", "1"), "stream_cpasync": ("0", "1", "0"),
-                                 "stream_ring": ("0", "0", "0")}.items():
-        os.environ["RL_XENC_RESIDENT"], os.environ["RL_XENC_CPASYNC"], os.environ["RL_XENC_MC"] = res, cpa, mc
-        Y.zero_()
-        assert lib.rl_xenc_linear(X.data_ptr(), img.data_ptr(), b.data_ptr(), Y.data_ptr(), T, N, K, act, s) == 0, lib.rl_last_error()
-        torch.cuda.synchronize()
-        err = (Y[:4096].float() - ref).abs().max().item()
-        tail_err = (Y[-128:].float() - (torch.nn.functional.gelu(X[-128:].float() @ W.half().float().T + b) if act
-                                        else X[-128:].float() @ W.half().float().T + b)).abs().max().item()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        for _ in range(3):
-            lib.rl_xenc_linear(X.data_ptr(), img.data_ptr(), b.data_ptr(), Y.data_ptr(), T, N, K, act, s)
-        e0.record()
-        for _ in range(20):
-            lib.rl_xenc_linear(X.data_ptr(), img.data_ptr(), b.data_ptr(), Y.data_ptr(), T, N, K, act, s)
-        e1.record()
-        torch.cuda.synchronize()
-        us = e0.elapsed_time(e1) / 20 * 1e3
-        out[f"{name}_{mode}"] = {"us": round(us, 1), "tflops": round(2.0 * T * N * K / us / 1e6, 1), "max_err": err,
-                                     "tail_err": tail_err}
+    Y.zero_()
+    assert lib.rl_xenc_linear(X.data_ptr(), img.data_ptr(), b.data_ptr(), Y.data_ptr(), T, N, K, act, s) == 0, lib.rl_last_error()
+    torch.cuda.synchronize()
+    err = (Y[:4096].float() - ref).abs().max().item()
+    tail_err = (Y[-128:].float() - (torch.nn.functional.gelu(X[-128:].float() @ W.half().float().T + b) if act
+                                    else X[-128:].float() @ W.half().float().T + b)).abs().max().item()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    for _ in range(3):
+        lib.rl_xenc_linear(X.data_ptr(), img.data_ptr(), b.data_ptr(), Y.data_ptr(), T, N, K, act, s)
+    e0.record()
+    for _ in range(20):
+        lib.rl_xenc_linear(X.data_ptr(), img.data_ptr(), b.data_ptr(), Y.data_ptr(), T, N, K, act, s)
+    e1.record()
+    torch.cuda.synchronize()
+    us = e0.elapsed_time(e1) / 20 * 1e3
+    out[name] = {"us": round(us, 1), "tflops": round(2.0 * T * N * K / us / 1e6, 1), "max_err": err, "tail_err": tail_err}
 print(json.dumps(out))
