@@ -291,8 +291,8 @@ typedef struct rl_xenc_weights {
   const rl_xenc_layer* layers; /* HOST array of n_layers entries */
   const float* pooler_w; /* fp32 [H, H] */
   const float* pooler_b;
-  const float* cls_w;    /* fp32 [H] (num_labels == 1) */
-  const float* cls_b;    /* fp32 [1] */
+  const float* cls_w;    /* fp32 [H]: the classifier row whose sigmoid is the score (row 1 of a two-label head) */
+  const float* cls_b;    /* fp32 [1]: that row's bias */
 } rl_xenc_weights;
 
 size_t rl_xenc_linear_image_bytes(int N, int K);
@@ -304,7 +304,8 @@ int rl_xenc_linear(const void* X, const void* image, const float* bias, void* Y,
                    void* stream);
 size_t rl_xenc_workspace_bytes(const rl_xenc_weights* w, int T);
 /* Packed variable-length batch: input_ids/type_ids/pos_ids [T], cu_seqlens [P+1]; max_len = longest
- * sequence.  out_logit[P], out_score[P] = sigmoid(logit) (FlashRank's score). */
+ * sequence.  out_logit[P], out_score[P] = sigmoid(logit) (FlashRank's score).  head_dim (hidden / n_heads)
+ * must be 32 or 64 and hidden a multiple of 32 up to 768; anything else returns RL_EUNSUPPORTED. */
 int rl_xenc_score(const rl_xenc_weights* w, const int32_t* input_ids, const int32_t* type_ids, const int32_t* pos_ids,
                   const int32_t* cu_seqlens, int P, int T, int max_len, float* out_logit, float* out_score,
                   void* workspace, size_t workspace_bytes, void* stream);

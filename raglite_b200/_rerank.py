@@ -55,9 +55,16 @@ class ScoreFnRanker:
         return RankedResults(results, query)
 
 
+# Where the Hugging Face weights of the default rerankers (RAGLiteConfig) come from.  FlashRank's
+# ms-marco-MultiBERT-L-12 is an ONNX export with no known Hugging Face twin, so none is named for it.
+HF_SOURCES = {"ms-marco-MiniLM-L-12-v2": "cross-encoder/ms-marco-MiniLM-L-12-v2"}
+
+
 class B200CrossEncoderRanker(ScoreFnRanker):
-    """BERT cross-encoder (ms-marco-MiniLM-L-12-v2 architecture) scored on the GPU.  Weights are
-    loaded lazily from ``cache_dir/<model_name>`` (HF ``safetensors`` + tokenizer files)."""
+    """BERT cross-encoder scored on the GPU: any ``BertForSequenceClassification`` with head_dim 32 or 64 and
+    hidden size up to 768, which covers both default rerankers (ms-marco-MiniLM-L-12-v2, H=384, and the BERT-base
+    ms-marco-MultiBERT-L-12, H=768).  Weights are loaded lazily from ``cache_dir/<model_name>`` (HF
+    ``config.json`` + ``safetensors`` + ``tokenizer.json``)."""
 
     def __init__(self, model_name: str, *, cache_dir: Path | str | None = None, max_length: int = 512,
                  device: Any | None = None):
@@ -74,11 +81,13 @@ class B200CrossEncoderRanker(ScoreFnRanker):
 
             path = (self.cache_dir / self.model_name) if self.cache_dir else Path(self.model_name)
             if not (path / "config.json").exists():
+                source = HF_SOURCES.get(self.model_name)
+                where = (f"e.g. `huggingface-cli download {source} --local-dir {path}`" if source else
+                         "a BERT-base-style BertForSequenceClassification directory converted from the model")
                 raise FileNotFoundError(
                     f"B200CrossEncoderRanker: no Hugging Face model directory at {path}.  The reference's FlashRank "
                     "reranker downloads an ONNX file on first use; this ranker needs the same model as HF weights "
-                    "(config.json + model.safetensors + tokenizer.json, e.g. `huggingface-cli download "
-                    f"cross-encoder/{self.model_name} --local-dir {path}`), or pass any object with a "
+                    f"(config.json + model.safetensors + tokenizer.json; {where}), or pass any object with a "
                     ".rank(query=, docs=) method as RAGLiteConfig.reranker (None disables reranking).  See INTEGRATION.md.")
             self._engine = CrossEncoderEngine.from_pretrained(path, max_length=self.max_length, device=self.device)
         return self._engine.score_pairs([query] * len(docs), list(docs))

@@ -2,7 +2,8 @@
 
 The reference calls ``reranker.rank(query=, docs=)`` (``_search.py:395``) on a ``rerankers``
 FlashRankRanker: tokenise (query, passage) pairs, run ms-marco-MiniLM-L-12-v2 (BERT, 12 layers, H=384,
-12 heads, FFN=1536) with onnxruntime, sigmoid the logit, sort.  Here the forward runs in
+12 heads, FFN=1536) or ms-marco-MultiBERT-L-12 (BERT-base: H=768, 12 heads of 64, FFN=3072, two labels)
+with onnxruntime, sigmoid the logit, sort.  Here the forward runs in
 ``rl_xenc_score`` (hand-written CUDA: tcgen05 linear layers with fused bias/GELU, attention,
 LayerNorm, pooler+classifier) on packed variable-length batches -- no padding tokens are computed.
 """
@@ -27,9 +28,10 @@ def _stream() -> int:
 
 
 def random_minilm_state_dict(seed: int = 0, *, n_layers: int = 12, hidden: int = 384, ffn: int = 1536,
-                             vocab: int = 30522, max_pos: int = 512) -> dict[str, torch.Tensor]:
+                             vocab: int = 30522, max_pos: int = 512, n_labels: int = 1) -> dict[str, torch.Tensor]:
     """Seeded random weights with the HF ``BertForSequenceClassification`` names/shapes of
-    ms-marco-MiniLM-L-12-v2 (real weights cannot be downloaded offline); for benchmarks and smoke tests."""
+    ms-marco-MiniLM-L-12-v2 (real weights cannot be downloaded offline); for benchmarks and smoke tests.
+    ``hidden=768, ffn=3072, vocab=105879, n_labels=2`` gives the shapes of ms-marco-MultiBERT-L-12."""
     g = torch.Generator().manual_seed(seed)
 
     def w(*shape: int) -> torch.Tensor:
@@ -41,7 +43,7 @@ def random_minilm_state_dict(seed: int = 0, *, n_layers: int = 12, hidden: int =
         "bert.embeddings.token_type_embeddings.weight": w(2, hidden),
         "bert.embeddings.LayerNorm.weight": torch.ones(hidden), "bert.embeddings.LayerNorm.bias": torch.zeros(hidden),
         "bert.pooler.dense.weight": w(hidden, hidden), "bert.pooler.dense.bias": torch.zeros(hidden),
-        "classifier.weight": w(1, hidden) * 8.0, "classifier.bias": torch.zeros(1),
+        "classifier.weight": w(n_labels, hidden) * 8.0, "classifier.bias": torch.zeros(n_labels),
     }
     for l in range(n_layers):
         p = f"bert.encoder.layer.{l}."
@@ -55,8 +57,24 @@ def random_minilm_state_dict(seed: int = 0, *, n_layers: int = 12, hidden: int =
     return sd
 
 
+def classifier_row(weight: torch.Tensor, bias: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
+    """The classifier row and bias whose sigmoid is FlashRank's score: column 0 of a one-label model, column 1
+    of a model with more labels (FlashRank scores ``sigmoid(logits[:, 1])`` then).  Returns ``([H], [1])``."""
+    weight = weight.detach()
+    weight = weight.reshape(1, -1) if weight.dim() == 1 else weight
+    bias = bias.detach().reshape(-1)
+    if weight.shape[0] != bias.numel() or weight.shape[0] < 1:
+        raise ValueError(f"classifier weight {tuple(weight.shape)} and bias {tuple(bias.shape)} do not match")
+    col = 1 if weight.shape[0] > 1 else 0
+    return weight[col].contiguous(), bias[col:col + 1].contiguous()
+
+
 class CrossEncoderEngine:
-    """Device-resident packed weights + tokenizer + batching."""
+    """Device-resident packed weights + tokenizer + batching.
+
+    Geometries: head_dim 32 or 64 and hidden a multiple of 32 up to 768 (MiniLM-L12-H384 and BERT-base).  The
+    classifier may have any number of labels; the engine keeps the one FlashRank scores (``classifier_row``), so
+    the returned ``logit`` is that column (``logits[:, 1]`` of a two-label model) and ``score`` its sigmoid."""
 
     def __init__(self, state_dict: dict[str, torch.Tensor], *, n_layers: int, hidden: int, n_heads: int, ffn: int,
                  max_pos: int, ln_eps: float = 1e-12, tokenizer: Any | None = None, max_length: int = 512,
@@ -116,10 +134,11 @@ class CrossEncoderEngine:
         w.emb_ln_g, w.emb_ln_b = f32("embeddings.LayerNorm.weight").data_ptr(), f32("embeddings.LayerNorm.bias").data_ptr()
         w.layers = C.cast(self._layers, C.POINTER(XencLayer))
         w.pooler_w, w.pooler_b = f32("pooler.dense.weight").data_ptr(), f32("pooler.dense.bias").data_ptr()
-        cls_w = state_dict["classifier.weight"].detach().to(device=self.device, dtype=torch.float32).reshape(-1).contiguous()
+        cls_w, cls_b = classifier_row(state_dict["classifier.weight"], state_dict["classifier.bias"])
         if cls_w.numel() != hidden:
-            raise ValueError("only single-logit classifiers (num_labels == 1) are supported")
-        cls_b = state_dict["classifier.bias"].detach().to(device=self.device, dtype=torch.float32).contiguous()
+            raise ValueError(f"classifier rows have {cls_w.numel()} columns, the model's hidden size is {hidden}")
+        cls_w = cls_w.to(device=self.device, dtype=torch.float32).contiguous()
+        cls_b = cls_b.to(device=self.device, dtype=torch.float32).contiguous()
         self._keep += [cls_w, cls_b]
         w.cls_w, w.cls_b = cls_w.data_ptr(), cls_b.data_ptr()
         self.weights = w
@@ -131,7 +150,7 @@ class CrossEncoderEngine:
     # ---- constructors ------------------------------------------------------------------------------
     @classmethod
     def from_hf(cls, model: Any, tokenizer: Any | None = None, **kw: Any) -> "CrossEncoderEngine":
-        """From a ``transformers.BertForSequenceClassification`` (num_labels == 1)."""
+        """From a ``transformers.BertForSequenceClassification`` (any ``num_labels``, see ``classifier_row``)."""
         c = model.config
         return cls(model.state_dict(), n_layers=c.num_hidden_layers, hidden=c.hidden_size, n_heads=c.num_attention_heads,
                    ffn=c.intermediate_size, max_pos=c.max_position_embeddings, ln_eps=c.layer_norm_eps,

@@ -1,4 +1,4 @@
-// BERT cross-encoder forward (ms-marco-MiniLM-L-12 architecture) for sm_100a: the arithmetic behind
+// BERT cross-encoder forward (ms-marco-MiniLM-L-12 and BERT-base geometries) for sm_100a: the arithmetic behind
 // rerank_chunks (reference _search.py:364-397 -> rerankers FlashRankRanker -> onnxruntime, all
 // third-party).  Variable-length packed batches (no padding): tokens [T, H], cu_seqlens [P + 1].
 //
@@ -7,7 +7,8 @@
 //                        sliced by 64), X copied into 128B-swizzled smem by loader warps, W as a
 //                        pre-swizzled fp16 image fetched with cp.async.bulk, fp32 accumulate in TMEM,
 //                        bias / GELU(erf) fused in the TMEM epilogue
-//   attention2_kernel    softmax(Q K^T / sqrt(dh)) V per (sequence, head), fp32 math
+//   attention2_kernel    softmax(Q K^T / sqrt(dh)) V per (sequence, head), fp32 math, head_dim 32
+//   attention64_kernel   the same for head_dim 64 (BERT-base), K / V streamed through a cp.async ring
 //   add_ln_kernel        LayerNorm(x + residual)
 //   cls_head_kernel      pooler (dense + tanh on [CLS]) -> classifier -> logit, sigmoid score
 #include <cuda.h>
@@ -533,6 +534,8 @@ __global__ void __launch_bounds__(kResThreads, 1) linear_wres_kernel(const __gri
 }
 
 // ---- embeddings + LayerNorm: one warp per token ----------------------------------------------------------
+// NC columns per lane: 16 for H <= 512 (MiniLM, H = 384), 24 for H <= 768 (BERT-base).
+template <int NC>
 __global__ void __launch_bounds__(256) embed_ln_kernel(const int32_t* __restrict__ ids, const int32_t* __restrict__ type_ids,
                                                        const int32_t* __restrict__ pos_ids, const __half* __restrict__ word,
                                                        const __half* __restrict__ pos, const __half* __restrict__ type,
@@ -546,10 +549,10 @@ __global__ void __launch_bounds__(256) embed_ln_kernel(const int32_t* __restrict
   const __half* w = word + (size_t)min(max(ids[tok], 0), vocab - 1) * H;
   const __half* p = pos + (size_t)min(max(pos_ids[tok], 0), max_pos - 1) * H;
   const __half* ty = type + (size_t)min(max(type_ids[tok], 0), type_vocab - 1) * H;
-  float x[16];  // H <= 512
+  float x[NC];  // H <= 32 NC
   float s = 0.f;
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
+  for (int i = 0; i < NC; ++i) {
     const int c = lane + 32 * i;
     x[i] = c < H ? __half2float(w[c]) + __half2float(p[c]) + __half2float(ty[c]) : 0.f;
     s += x[i];
@@ -557,13 +560,13 @@ __global__ void __launch_bounds__(256) embed_ln_kernel(const int32_t* __restrict
   const float mean = warp_sum_f(s) / (float)H;
   float var = 0.f;
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
+  for (int i = 0; i < NC; ++i) {
     const int c = lane + 32 * i;
     if (c < H) var += (x[i] - mean) * (x[i] - mean);
   }
   const float rstd = rsqrtf(warp_sum_f(var) / (float)H + eps);
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
+  for (int i = 0; i < NC; ++i) {
     const int c = lane + 32 * i;
     if (c < H) out[(size_t)tok * H + c] = __float2half_rn((x[i] - mean) * rstd * g[c] + bta[c]);
   }
@@ -571,21 +574,24 @@ __global__ void __launch_bounds__(256) embed_ln_kernel(const int32_t* __restrict
 
 // out = LayerNorm(x + res), one warp per token.  H % 128 == 0 (384 for MiniLM): a lane owns the columns
 // lane * 4 + 128 i, so every load / store instruction of the warp covers 256 contiguous bytes (8-byte pieces);
-// the first version moved 2 bytes per lane and instruction and ran at 3.5 TB/s.
-template <bool VEC>
+// the first version moved 2 bytes per lane and instruction and ran at 3.5 TB/s.  NC columns per lane as in
+// embed_ln_kernel: H <= 32 NC (VEC: NC / 4 pieces of 128 columns).
+template <bool VEC, int NC>
 __global__ void __launch_bounds__(256) add_ln_kernel(const __half* __restrict__ xin, const __half* __restrict__ res,
                                                      const float* __restrict__ g, const float* __restrict__ bta, float eps,
                                                      int T, int H, __half* __restrict__ out) {
   const int lane = threadIdx.x & 31;
   const int tok = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (tok >= T) return;
-  float x[16];   // H <= 512
+  static_assert(NC % 4 == 0, "VEC pieces hold four columns per lane");
+  constexpr int NP = NC / 4;   // 128-column pieces (VEC)
+  float x[NC];   // H <= 32 NC
   float s = 0.f;
   if (VEC) {
     const uint2* xi = reinterpret_cast<const uint2*>(xin + (size_t)tok * H);
     const uint2* ri = reinterpret_cast<const uint2*>(res + (size_t)tok * H);
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < NP; ++i) {
       if (i * 128 < H) {
         const uint2 a = __ldg(xi + lane + 32 * i), r = __ldg(ri + lane + 32 * i);
         const float2 a0 = __half22float2(*reinterpret_cast<const __half2*>(&a.x)), a1 = __half22float2(*reinterpret_cast<const __half2*>(&a.y));
@@ -598,7 +604,7 @@ __global__ void __launch_bounds__(256) add_ln_kernel(const __half* __restrict__ 
     }
   } else {
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
+    for (int i = 0; i < NC; ++i) {
       const int c = lane + 32 * i;
       x[i] = c < H ? __half2float(xin[(size_t)tok * H + c]) + __half2float(res[(size_t)tok * H + c]) : 0.f;
       s += x[i];
@@ -607,7 +613,7 @@ __global__ void __launch_bounds__(256) add_ln_kernel(const __half* __restrict__ 
   const float mean = warp_sum_f(s) / (float)H;
   float var = 0.f;
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
+  for (int i = 0; i < NC; ++i) {
     const int c = VEC ? (i >> 2) * 128 : lane + 32 * i;   // (VEC: all four values of a piece are in or out together)
     if (c < H) var += (x[i] - mean) * (x[i] - mean);
   }
@@ -615,7 +621,7 @@ __global__ void __launch_bounds__(256) add_ln_kernel(const __half* __restrict__ 
   if (VEC) {
     uint2* oo = reinterpret_cast<uint2*>(out + (size_t)tok * H);
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int i = 0; i < NP; ++i) {
       if (i * 128 < H) {
         const float4 gg = __ldg(reinterpret_cast<const float4*>(g) + lane + 32 * i);
         const float4 bb = __ldg(reinterpret_cast<const float4*>(bta) + lane + 32 * i);
@@ -627,7 +633,7 @@ __global__ void __launch_bounds__(256) add_ln_kernel(const __half* __restrict__ 
     }
   } else {
 #pragma unroll
-    for (int i = 0; i < 16; ++i) {
+    for (int i = 0; i < NC; ++i) {
       const int c = lane + 32 * i;
       if (c < H) out[(size_t)tok * H + c] = __float2half_rn((x[i] - mean) * rstd * g[c] + bta[c]);
     }
@@ -872,6 +878,171 @@ __global__ void __launch_bounds__(128, 3) attention2_kernel(const __half* __rest
   }
 }
 
+// ---- attention for head_dim 64 (BERT-base: 12 heads x 64) ------------------------------------------------
+// Same math as attention2_kernel (m16n8k16 fp16 MMAs, fp32 accumulate, online softmax in the exp2 domain) and the same
+// launch order (one CTA per (sequence, head), heads fastest, sequences longest first).  Two things differ, both forced
+// by the wider head:
+//   - One 16-query tile per warp.  O (32 registers), the Q fragments (16) and the scores of a 64-key block (32) fit the
+//     168-register cap of three CTAs per SM; two tiles per warp would need 160 for these alone and spill.  (At four
+//     CTAs per SM, a 128-register cap, ptxas spills 16 bytes.)
+//   - K and V stream through shared memory in 64-key blocks, double-buffered with cp.async, instead of staying
+//     resident: a whole 512-token head at a 144-byte pitch is 147 KB, one CTA per SM.  The ring is 36 KB whatever the
+//     sequence length.
+// The CTA walks its queries in passes of 64 (warp w owns queries [64 p + 16 w, + 16)) and streams the head's keys once
+// per pass; the block stream runs across passes, so the next pass's first block loads while this pass ends.  The last
+// block of a pass is 16, 32 or 64 keys wide (the fewest that cover the keys left).
+constexpr int kAtt64Pitch = 72;    // halves per staged key row: 144 bytes, conflict-free ldmatrix
+constexpr int kAtt64Keys = 64;     // keys per streamed block
+constexpr int kAtt64StageHalves = 2 * kAtt64Keys * kAtt64Pitch;   // K rows, then V rows
+constexpr int kAtt64Stages = 2;
+
+__global__ void __launch_bounds__(128, 3) attention64_kernel(const __half* __restrict__ qkv, const int32_t* __restrict__ cu,
+                                                          const int32_t* __restrict__ order, int H, int n_heads,
+                                                          float scale_log2e, __half* __restrict__ ctx) {
+  __shared__ __align__(16) __half kv_smem[kAtt64Stages * kAtt64StageHalves];   // 36 864 bytes
+  const int head = (int)(blockIdx.x % (unsigned)n_heads);
+  const int seq = order[blockIdx.x / (unsigned)n_heads];
+  const int t0 = cu[seq], L = cu[seq + 1] - t0;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const size_t ld = (size_t)3 * H;
+  const int n_kb = (L + kAtt64Keys - 1) / kAtt64Keys;   // key blocks per pass
+  const int n_blocks = (L + 63) / 64 * n_kb;            // passes x key blocks
+  // Block g -> stage g % 2: K and V rows of keys [64 (g % n_kb), + 64), zero-filled past the sequence.
+  auto load_block = [&](int g) {
+    const int kb = (g % n_kb) * kAtt64Keys;
+    __half* Ks = kv_smem + (g & 1) * kAtt64StageHalves;
+    __half* Vs = Ks + kAtt64Keys * kAtt64Pitch;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {   // 64 keys x 8 16-byte chunks of K and of V, 128 threads
+      const int idx = threadIdx.x + 128 * i;
+      const int j = idx >> 3, c = idx & 7;
+      const int key = kb + j;
+      const __half* src = qkv + (size_t)(t0 + (key < L ? key : L - 1)) * ld + head * 64 + c * 8;
+      const uint32_t nbytes = key < L ? 16u : 0u;
+      cp_async_16(smem_u32(Ks + j * kAtt64Pitch + c * 8), src + H, nbytes);
+      cp_async_16(smem_u32(Vs + j * kAtt64Pitch + c * 8), src + 2 * H, nbytes);
+    }
+  };
+  const int r = lane >> 2, cp = (lane & 3) * 2;
+  uint32_t a[4][4];   // Q fragments of the warp's tile (rows >= L read as zero)
+  float m[2] = {-INFINITY, -INFINITY}, l[2] = {0.f, 0.f}, O[8][4];
+  // One key block of NKK k-steps (16 keys each); NKK is a compile-time constant so that the loops unroll without guards.
+  auto block = [&](auto nkk_tag, const __half* Ks, const __half* Vs, int kb) {
+    constexpr int NKK = decltype(nkk_tag)::value;
+    constexpr int NJ = 2 * NKK;   // 8-key score tiles
+    float S[NJ][4];
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) {
+      uint32_t b[4], b2[4];
+      ldsm_x4(b, Ks + (j * 8 + (lane & 7)) * kAtt64Pitch + (lane >> 3) * 8);          // dims 0..31
+      ldsm_x4(b2, Ks + (j * 8 + (lane & 7)) * kAtt64Pitch + 32 + (lane >> 3) * 8);    // dims 32..63
+#pragma unroll
+      for (int e = 0; e < 4; ++e) S[j][e] = 0.f;
+      mma16816(S[j], a[0], b[0], b[1]);
+      mma16816(S[j], a[1], b[2], b[3]);
+      mma16816(S[j], a[2], b2[0], b2[1]);
+      mma16816(S[j], a[3], b2[2], b2[3]);
+    }
+    if (kb + NJ * 8 > L) {   // only the last key block holds padding keys
+#pragma unroll
+      for (int j = 0; j < NJ; ++j)
+#pragma unroll
+        for (int e = 0; e < 4; ++e)
+          if (kb + j * 8 + cp + (e & 1) >= L) S[j][e] = -INFINITY;
+    }
+    float mx0 = -INFINITY, mx1 = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < NJ; ++j) {
+      mx0 = fmaxf(mx0, fmaxf(S[j][0], S[j][1]));
+      mx1 = fmaxf(mx1, fmaxf(S[j][2], S[j][3]));
+    }
+    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 1));
+    mx0 = fmaxf(mx0, __shfl_xor_sync(0xffffffffu, mx0, 2));
+    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 1));
+    mx1 = fmaxf(mx1, __shfl_xor_sync(0xffffffffu, mx1, 2));
+    // finite: every block holds at least one valid key (kb < L)
+    const float mn0 = fmaxf(m[0], mx0 * scale_log2e), mn1 = fmaxf(m[1], mx1 * scale_log2e);
+    const float c0 = ex2_approx(m[0] - mn0), c1 = ex2_approx(m[1] - mn1);
+    l[0] *= c0; l[1] *= c1;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { O[i][0] *= c0; O[i][1] *= c0; O[i][2] *= c1; O[i][3] *= c1; }
+    m[0] = mn0; m[1] = mn1;
+#pragma unroll
+    for (int j = 0; j < NJ; ++j)
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float pexp = ex2_approx(fmaf(S[j][e], scale_log2e, e < 2 ? -mn0 : -mn1));   // -inf -> 0
+        S[j][e] = pexp;
+        if (e < 2) l[0] += pexp; else l[1] += pexp;
+      }
+#pragma unroll
+    for (int kk = 0; kk < NKK; ++kk) {
+      uint32_t pa[4];
+      pa[0] = pack_half2(S[2 * kk][0], S[2 * kk][1]);
+      pa[1] = pack_half2(S[2 * kk][2], S[2 * kk][3]);
+      pa[2] = pack_half2(S[2 * kk + 1][0], S[2 * kk + 1][1]);
+      pa[3] = pack_half2(S[2 * kk + 1][2], S[2 * kk + 1][3]);
+#pragma unroll
+      for (int dn2 = 0; dn2 < 4; ++dn2) {
+        uint32_t vb[4];
+        ldsm_x4_trans(vb, Vs + (kk * 16 + (lane & 7) + ((lane >> 3) & 1) * 8) * kAtt64Pitch + (dn2 * 2 + (lane >> 4)) * 8);
+        mma16816(O[dn2 * 2], pa, vb[0], vb[1]);
+        mma16816(O[dn2 * 2 + 1], pa, vb[2], vb[3]);
+      }
+    }
+  };
+  if (n_blocks > 0) load_block(0);
+  asm volatile("cp.async.commit_group;" ::: "memory");
+  for (int g = 0; g < n_blocks; ++g) {
+    const int pass = g / n_kb, kbi = g - pass * n_kb, kb = kbi * kAtt64Keys;
+    if (g + 1 < n_blocks) load_block(g + 1);
+    asm volatile("cp.async.commit_group;" ::: "memory");   // (an empty group at the end keeps the wait below uniform)
+    const int q0 = pass * 64 + warp * 16 + r, q1 = q0 + 8;
+    const bool active = pass * 64 + warp * 16 < L;   // warp-uniform: the tile holds at least one query
+    if (active && kbi == 0) {   // a new pass: this warp's Q fragments and a fresh softmax state
+#pragma unroll
+      for (int ks = 0; ks < 4; ++ks) {
+        const __half* p0 = qkv + (size_t)(t0 + q0) * ld + head * 64 + ks * 16 + cp;
+        const __half* p1 = qkv + (size_t)(t0 + q1) * ld + head * 64 + ks * 16 + cp;
+        a[ks][0] = q0 < L ? __ldg(reinterpret_cast<const uint32_t*>(p0)) : 0u;
+        a[ks][1] = q1 < L ? __ldg(reinterpret_cast<const uint32_t*>(p1)) : 0u;
+        a[ks][2] = q0 < L ? __ldg(reinterpret_cast<const uint32_t*>(p0 + 8)) : 0u;
+        a[ks][3] = q1 < L ? __ldg(reinterpret_cast<const uint32_t*>(p1 + 8)) : 0u;
+      }
+      m[0] = m[1] = -INFINITY;
+      l[0] = l[1] = 0.f;
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+#pragma unroll
+        for (int e = 0; e < 4; ++e) O[i][e] = 0.f;
+    }
+    asm volatile("cp.async.wait_group 1;" ::: "memory");   // block g has landed (this thread's copies) ...
+    __syncthreads();                                        // ... and every thread's
+    if (active) {
+      const __half* Ks = kv_smem + (g & 1) * kAtt64StageHalves;
+      const __half* Vs = Ks + kAtt64Keys * kAtt64Pitch;
+      const int rem = L - kb;
+      if (rem > 32) block(std::integral_constant<int, 4>{}, Ks, Vs, kb);
+      else if (rem > 16) block(std::integral_constant<int, 2>{}, Ks, Vs, kb);
+      else block(std::integral_constant<int, 1>{}, Ks, Vs, kb);
+      if (kbi == n_kb - 1) {   // the pass is done: normalise and store this warp's 16 rows
+        float s0 = l[0], s1 = l[1];
+        s0 += __shfl_xor_sync(0xffffffffu, s0, 1);
+        s0 += __shfl_xor_sync(0xffffffffu, s0, 2);
+        s1 += __shfl_xor_sync(0xffffffffu, s1, 1);
+        s1 += __shfl_xor_sync(0xffffffffu, s1, 2);
+        const float inv0 = 1.f / s0, inv1 = 1.f / s1;
+#pragma unroll
+        for (int dn = 0; dn < 8; ++dn) {
+          if (q0 < L) *reinterpret_cast<uint32_t*>(ctx + (size_t)(t0 + q0) * H + head * 64 + dn * 8 + cp) = pack_half2(O[dn][0] * inv0, O[dn][1] * inv0);
+          if (q1 < L) *reinterpret_cast<uint32_t*>(ctx + (size_t)(t0 + q1) * H + head * 64 + dn * 8 + cp) = pack_half2(O[dn][2] * inv1, O[dn][3] * inv1);
+        }
+      }
+    }
+    __syncthreads();   // stage g % 2 is free for block g + 2
+  }
+}
+
 // ---- pooler + classifier ----------------------------------------------------------------------------------
 // logit[s] = Wc . tanh(Wp h_s + bp) + bc with h_s the [CLS] row of sequence s.  A CTA owns kClsSeqs sequences
 // (their [CLS] rows sit in shared memory as fp32) and its H/32 warps share the H pooler outputs; for one output
@@ -1054,8 +1225,10 @@ extern "C" int rl_xenc_score(const rl_xenc_weights* w, const int32_t* input_ids,
              "rl_xenc_score: null pointer");
   if (P == 0 || T == 0) return RL_OK;
   const int H = w->hidden, F = w->ffn, nh = w->n_heads;
-  RL_REQUIRE(H % 32 == 0 && H <= 512 && nh > 0 && H / nh == 32, RL_EUNSUPPORTED,
-             "rl_xenc_score: hidden=%d heads=%d unsupported (head_dim must be 32, hidden <= 512)", H, nh);
+  const int head_dim = nh > 0 && H % nh == 0 ? H / nh : 0;
+  RL_REQUIRE(H % 32 == 0 && H > 0 && H <= 768 && (head_dim == 32 || head_dim == 64), RL_EUNSUPPORTED,
+             "rl_xenc_score: hidden=%d heads=%d unsupported (supported: head_dim 32 or 64, hidden a multiple of 32 up to 768)",
+             H, nh);
   RL_REQUIRE(F % 32 == 0 && max_len > 0 && max_len <= w->max_pos, RL_EUNSUPPORTED, "rl_xenc_score: bad ffn / max_len");
   RL_REQUIRE(workspace && workspace_bytes >= rl_xenc_workspace_bytes(w, T), RL_ENOSPACE, "rl_xenc_score: workspace too small");
   int dev = 0, sms = 148;
@@ -1074,33 +1247,49 @@ extern "C" int rl_xenc_score(const rl_xenc_weights* w, const int32_t* input_ids,
   RL_CUDA_CHECK(cudaGetLastError());
   const int tok_blocks = (T + 7) / 8;
   const bool ln_vec = H % 128 == 0;   // (LayerNorm gamma / beta come from torch allocations: 16-byte aligned)
-  embed_ln_kernel<<<tok_blocks, 256, 0, stream>>>(input_ids, type_ids, pos_ids, reinterpret_cast<const __half*>(w->word_emb),
-                                                  reinterpret_cast<const __half*>(w->pos_emb),
-                                                  reinterpret_cast<const __half*>(w->type_emb), w->emb_ln_g, w->emb_ln_b,
-                                                  w->ln_eps, T, H, w->vocab, w->max_pos, w->type_vocab, hidden);
+  const bool ln_wide = H > 512;       // 24 columns per lane instead of 16
+  const __half* word_emb = reinterpret_cast<const __half*>(w->word_emb);
+  const __half* pos_emb = reinterpret_cast<const __half*>(w->pos_emb);
+  const __half* type_emb = reinterpret_cast<const __half*>(w->type_emb);
+  if (ln_wide)
+    embed_ln_kernel<24><<<tok_blocks, 256, 0, stream>>>(input_ids, type_ids, pos_ids, word_emb, pos_emb, type_emb, w->emb_ln_g,
+                                                        w->emb_ln_b, w->ln_eps, T, H, w->vocab, w->max_pos, w->type_vocab, hidden);
+  else
+    embed_ln_kernel<16><<<tok_blocks, 256, 0, stream>>>(input_ids, type_ids, pos_ids, word_emb, pos_emb, type_emb, w->emb_ln_g,
+                                                        w->emb_ln_b, w->ln_eps, T, H, w->vocab, w->max_pos, w->type_vocab, hidden);
   RL_CUDA_CHECK(cudaGetLastError());
-  const size_t att_smem = (size_t)((max_len + 63) / 64 * 64) * kAttPitch * 2 * sizeof(__half);
-  RL_REQUIRE(att_smem <= 200 * 1024, RL_EUNSUPPORTED, "rl_xenc_score: max_len=%d too long for the attention kernel", max_len);
-  RL_CUDA_CHECK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem));
-  const float scale = 1.4426950408889634f / sqrtf(32.f);  // softmax in the exp2 domain
+  auto add_ln = [&](const float* g, const float* b) {   // hidden = LayerNorm(tmp + hidden)
+    if (ln_wide && ln_vec) add_ln_kernel<true, 24><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, g, b, w->ln_eps, T, H, hidden);
+    else if (ln_wide) add_ln_kernel<false, 24><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, g, b, w->ln_eps, T, H, hidden);
+    else if (ln_vec) add_ln_kernel<true, 16><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, g, b, w->ln_eps, T, H, hidden);
+    else add_ln_kernel<false, 16><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, g, b, w->ln_eps, T, H, hidden);
+  };
+  size_t att_smem = 0;
+  if (head_dim == 32) {   // attention2_kernel stages the whole head; attention64_kernel streams it (static 36 KB)
+    att_smem = (size_t)((max_len + 63) / 64 * 64) * kAttPitch * 2 * sizeof(__half);
+    RL_REQUIRE(att_smem <= 200 * 1024, RL_EUNSUPPORTED, "rl_xenc_score: max_len=%d too long for the attention kernel", max_len);
+    RL_CUDA_CHECK(cudaFuncSetAttribute(attention2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)att_smem));
+  }
+  const float scale = 1.4426950408889634f / sqrtf((float)head_dim);  // softmax in the exp2 domain
   for (int l = 0; l < w->n_layers; ++l) {
     const rl_xenc_layer& L = w->layers[l];
     int rc = launch_linear(hidden, L.qkv_img, L.qkv_bias, qkv, T, 3 * H, H, 0, sms, stream);
     if (rc != RL_OK) return rc;
-    attention2_kernel<<<(unsigned)P * (unsigned)nh, 128, att_smem, stream>>>(qkv, cu_seqlens, seq_order, H, nh, scale, ctx,
-                                                                            P, /*seq_fastest=*/0, /*stage_async=*/1);
+    if (head_dim == 32)
+      attention2_kernel<<<(unsigned)P * (unsigned)nh, 128, att_smem, stream>>>(qkv, cu_seqlens, seq_order, H, nh, scale, ctx,
+                                                                              P, /*seq_fastest=*/0, /*stage_async=*/1);
+    else
+      attention64_kernel<<<(unsigned)P * (unsigned)nh, 128, 0, stream>>>(qkv, cu_seqlens, seq_order, H, nh, scale, ctx);
     RL_CUDA_CHECK(cudaGetLastError());
     rc = launch_linear(ctx, L.o_img, L.o_bias, tmp, T, H, H, 0, sms, stream);
     if (rc != RL_OK) return rc;
-    if (ln_vec) add_ln_kernel<true><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, L.ln1_g, L.ln1_b, w->ln_eps, T, H, hidden);
-    else add_ln_kernel<false><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, L.ln1_g, L.ln1_b, w->ln_eps, T, H, hidden);
+    add_ln(L.ln1_g, L.ln1_b);
     RL_CUDA_CHECK(cudaGetLastError());
     rc = launch_linear(hidden, L.up_img, L.up_bias, ffn, T, F, H, 1, sms, stream);
     if (rc != RL_OK) return rc;
     rc = launch_linear(ffn, L.down_img, L.down_bias, tmp, T, H, F, 0, sms, stream);
     if (rc != RL_OK) return rc;
-    if (ln_vec) add_ln_kernel<true><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, L.ln2_g, L.ln2_b, w->ln_eps, T, H, hidden);
-    else add_ln_kernel<false><<<tok_blocks, 256, 0, stream>>>(tmp, hidden, L.ln2_g, L.ln2_b, w->ln_eps, T, H, hidden);
+    add_ln(L.ln2_g, L.ln2_b);
     RL_CUDA_CHECK(cudaGetLastError());
   }
   const int cls_warps = H / 32 < kClsMaxWarps ? H / 32 : kClsMaxWarps;

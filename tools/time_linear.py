@@ -1,6 +1,8 @@
 """Cross-encoder linear layer as rl_xenc_linear dispatches it (weight-resident kernel for K <= 384, streaming
 kernel otherwise): parity of every GEMM shape against torch (incl. a ragged token count), then CUDA-event timing
-of back-to-back launches."""
+of back-to-back launches.  ``--bert-base`` times the BERT-base shapes (hidden 768, FFN 3072: ms-marco-MultiBERT-L-12)
+instead of the MiniLM ones."""
+import argparse
 import json
 import sys
 from pathlib import Path
@@ -14,7 +16,12 @@ from raglite_b200 import _lib  # noqa: E402
 lib = _lib.load()
 g = torch.Generator().manual_seed(0)
 T = 51200 + 77   # ragged: the last token tile is partial
+ap = argparse.ArgumentParser()
+ap.add_argument("--bert-base", action="store_true")
+args = ap.parse_args()
 shapes = [("qkv", 1152, 384, 0), ("out", 384, 384, 0), ("ffn_up", 1536, 384, 1), ("ffn_down", 384, 1536, 0)]
+if args.bert_base:
+    shapes = [("qkv", 2304, 768, 0), ("out", 768, 768, 0), ("ffn_up", 3072, 768, 1), ("ffn_down", 768, 3072, 0)]
 out = {}
 s = torch.cuda.current_stream().cuda_stream
 for name, N, K, act in shapes:
